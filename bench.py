@@ -6,6 +6,7 @@
     python bench.py --config 3 --total 8192 [--gpus N]                  # configs[2] as written: 8192 pictures, strong scaling
     python bench.py --config 4 --qpd6 0|4                               # configs[3]: 64 pictures 3840x2160 (split over ranks)
     python bench.py --config 5 --mode crop|xl                           # configs[4]: one 15991x11993 picture (one GPU)
+    python bench.py ... --dump-outputs DIR                              # also write the last timed step's outputs as .npy
 
 A "step" is one pass of the hot path over one batch.  Default: `--images` (1036 = 148 SMs x 7 pictures per CTA) synthetic
 768x512 pictures PER GPU at qpd6=2 -- a shard of BASELINE.json configs[2] (weak scaling: per-GPU work fixed; pictures are
@@ -188,6 +189,30 @@ def gate(dg, gold, base, where):
     return n_gold
 
 
+DUMP_RCON_BYTES, DUMP_STREAM_BYTES = 40 << 20, 20 << 20     # float32 payload; with the lengths the dump stays under 64 MB
+
+
+def dump_outputs(d, streams, rcons):
+    """--dump-outputs: what the caller of the timed path received from its last step, so that two builds can be compared
+    output for output.  stream_len.npy (float64) holds every picture's stream length.  For a sample of pictures drawn with
+    a fixed seed from the picture count and sizes alone (the same pictures whatever the build computes), rcon_NNNN.npy
+    holds the reconstruction and stream_NNNN.npy the stream bytes, both float32.  An array larger than its share of the
+    budget is written as every k-th element of its flattened form, k the smallest step that fits."""
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "stream_len.npy"), np.array([len(s) for s in streams], np.float64))
+    picks, px = [], 0
+    for i in np.random.default_rng(0).permutation(len(rcons)):
+        if picks and px + rcons[i].size > DUMP_RCON_BYTES // 4:
+            break
+        picks.append(int(i))
+        px += rcons[i].size
+    for i in picks:
+        for kind, a, room in (("rcon", rcons[i], DUMP_RCON_BYTES // 4),
+                              ("stream", np.frombuffer(bytes(streams[i]), np.uint8), DUMP_STREAM_BYTES // 4 // len(picks))):
+            k = max(1, -(-a.size // room))
+            np.save(os.path.join(d, f"{kind}_{i:04d}.npy"), (a if k == 1 else a.reshape(-1)[::k]).astype(np.float32))
+
+
 def run_one_call(a, H, WL, torch):
     """One process, one HEVCImageEncoderBatch call, N devices (hevce_api.c shards by CTU count, two chunk workers per device)."""
     nd = a.one_call
@@ -215,6 +240,8 @@ def run_one_call(a, H, WL, torch):
             s2, r2 = H.HEVCImageEncoderBatch(imgs, a.qpd6, outputs=host_out, copy_streams=False)
             t += time.perf_counter() - t0
             gate(digests(s2, r2), gold, base, "one-call arm")
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, s2, r2)
     px = n * KODAK_PIXELS
     v = px * a.steps / t / 1e6
     line = {
@@ -235,7 +262,7 @@ def run_one_call(a, H, WL, torch):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 3; --single-pass times exactly one)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", type=int, default=3, choices=[3, 4, 5])
@@ -245,6 +272,9 @@ def main():
     ap.add_argument("--qpd6", type=int, default=2)
     ap.add_argument("--cpu-sample", type=int, default=-1, help="pictures for the cpu_baseline leg (-1 = one per host core)")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the streams and reconstructions of the last one as DIR/<name>.npy "
+                         "(float32 / float64, under 64 MB: a fixed sample of the pictures; with several ranks, DIR/rank<r>/ each)")
     ap.add_argument("--one-call", type=int, default=0, metavar="N",
                     help="the library's own multi-GPU path: ONE process, ONE HEVCImageEncoderBatch call over N devices with N x --images "
                          "pictures (config 3); reports the end-to-end figure only (value = e2e)")
@@ -252,6 +282,11 @@ def main():
                     help="long single steps (configs 4-5): ONE upload + encode + download through the session calls that "
                          "HEVCImageEncoderBatch makes; value = the encode part, e2e = the whole pass, no warm-up")
     a = ap.parse_args()
+    if a.single_pass and a.steps not in (None, 1):
+        raise SystemExit("bench.py: --single-pass times exactly one step; drop --steps or pass --steps 1")
+    if a.dump_outputs and a.impl == "reference":
+        raise SystemExit("bench.py: --dump-outputs needs the GPU arms (the reference arm's batch is one picture per host core)")
+    a.steps = 3 if a.steps is None else a.steps
     if a.impl == "ours" and not a.single_pass:
         a.warmup = max(a.warmup, 3)
     if a.single_pass:
@@ -341,6 +376,8 @@ def main():
         last = digests(*out_last)
         n_gold = gate(last, gold, base, "device-resident arm, last timed step")
         base = base or last
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs if world == 1 else os.path.join(a.dump_outputs, f"rank{rank}"), *out_last)
         ses.close()
     value = pixels_step * a.steps / dt / 1e6
 

@@ -45,10 +45,6 @@ def ref():
     return _cache["ref"]
 
 
-def have_ref():
-    return os.path.exists(REF_SO) or os.path.exists("/root/reference/src/HEVCe.c")
-
-
 def oracle():
     if "oracle" not in _cache:
         _cache["oracle"] = _load(ORACLE_SO)
@@ -84,6 +80,21 @@ def oracle_encode(img, qpd6):
 
 def sha(b):
     return hashlib.sha256(bytes(b)).hexdigest()
+
+
+def report_figures(img, rcon, n):
+    """The result lines the reference CLI prints (HEVCeMain.c) for input `img`, reconstruction `rcon` and an n-byte
+    stream: sizes, ratio, bits per pixel, MSE over the overlap of the two sizes (floored at 1e-9) and PSNR."""
+    hp, wp = rcon.shape
+    hm, wm = min(img.shape[0], hp), min(img.shape[1], wp)
+    mse = max(float(((img[:hm, :wm].astype(np.int64) - rcon[:hm, :wm]) ** 2).sum()) / hm / wm, 1e-9)
+    return [f"  padded image size               = {wp} x {hp}",
+            f"  original   length               = {wp * hp} Bytes",
+            f"  compressed length               = {n} Bytes",
+            f"  compression ratio               = {wp * hp / n:.5f}",
+            f"  bits per pixel                  = {8.0 * n / (wp * hp):.5f}",
+            f"  mean square error (MSE)         = {mse:.7f}",
+            f"  peak signal/noise ratio (PSNR)  = {10.0 * np.log10(255 * 255 / mse):.4f} dB"]
 
 
 def read_pgm(path):

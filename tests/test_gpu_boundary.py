@@ -17,6 +17,7 @@ pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF_CLI = os.path.join(ROOT, "oracle", "_ref", "HEVCe")
 REF_MAIN_ON_US = os.path.join(ROOT, "oracle", "_ref", "HEVCeMain_on_b200")
+DROPIN_CLI = os.path.join(ROOT, "hevc-image-encoder-lite_b200", "HEVCe")
 
 
 @pytest.fixture(scope="module")
@@ -35,23 +36,32 @@ def write_pgm(path, img):
 
 @pytest.mark.parametrize("pic,q", [("k05", "2"), ("k19", "4")])
 def test_reference_main_runs_on_this_library(tmp_path, pic, q):
-    """HEVCeMain.c:197 calls HEVCImageEncoder; the binary below is that file, unmodified, linked against
-    libhevce_b200.so (oracle/Makefile).  Its .h265, reconstruction PGM and printed report must equal those of the
-    reference CLI built from the reference's own HEVCe.c -- on two full Kodak pictures (one landscape, one portrait)."""
-    if not (os.path.exists(REF_CLI) and os.path.exists(REF_MAIN_ON_US)):
-        pytest.skip("oracle/_ref binaries not built (they are made in the build container)")
-    imgs, _ = G.kodak()
+    """HEVCeMain.c:197 calls HEVCImageEncoder; HEVCeMain_on_b200 is that file, unmodified, linked against
+    libhevce_b200.so (oracle/Makefile), and hevc-image-encoder-lite_b200/HEVCe is the drop-in CLI.  On two full Kodak
+    pictures (one landscape, one portrait) each .h265 and reconstruction PGM must be the reference's (length and SHA-256
+    in the Kodak manifest) and each report must give the figures of that stream and reconstruction.  Where oracle/_ref
+    holds the reference CLI built from the reference's own sources, both must also equal its output byte for byte,
+    report included."""
+    imgs, man = G.kodak()
+    want = man[pic[1:]]["q"][q]
     src = tmp_path / "in.pgm"
     write_pgm(src, imgs[pic])
     outs = {}
-    for tag, exe in (("ref", REF_CLI), ("ours", REF_MAIN_ON_US)):
+    for tag, exe in (("ref", REF_CLI), ("ours", REF_MAIN_ON_US), ("dropin", DROPIN_CLI)):
+        if tag != "dropin" and not os.path.exists(exe):
+            continue
         h265, rec = tmp_path / f"{tag}.h265", tmp_path / f"{tag}.pgm"
         r = subprocess.run([exe, str(src), str(h265), q, str(rec)], capture_output=True, text=True, timeout=600)
         assert r.returncode == 0, r.stdout + r.stderr
         outs[tag] = (h265.read_bytes(), rec.read_bytes(), r.stdout.replace(str(h265), "<s>").replace(str(rec), "<r>"))
-    assert outs["ours"][0] == outs["ref"][0]
-    assert outs["ours"][1] == outs["ref"][1]
-    assert outs["ours"][2] == outs["ref"][2]
+        assert len(outs[tag][0]) == want["len"] and R.sha(outs[tag][0]) == want["stream_sha256"], tag
+        assert R.sha(outs[tag][1]) == want["rcon_pgm_sha256"], tag
+        report = outs[tag][2].splitlines()
+        for line in R.report_figures(imgs[pic], R.read_pgm(str(rec)), want["len"]):
+            assert line in report, (tag, line)
+    if "ref" in outs:
+        for tag in set(outs) - {"ref"}:
+            assert outs[tag] == outs["ref"], tag
 
 
 def test_concurrent_callers(H):

@@ -6,6 +6,7 @@ manifest of all 24 Kodak images x qpd6 0..4, whose qpd6=4 column is also checked
 shipped goldens testimage_out/NN.h265 when the manifest is generated (tools/make_golden.py).
 """
 import ctypes
+import json
 import os
 
 import numpy as np
@@ -55,10 +56,18 @@ def test_oracle_kodak_all(q):
 
 def test_generated_tables_match_reference_exports():
     """DCT/DST matrices, CABAC state tables, context init and scan orders are generated from the HEVC definitions
-    in the oracle; compare with the symbols the reference library exports (skipped where _ref is absent)."""
+    in the oracle; compare with the symbols the reference library exports.  Where oracle/_ref is absent, the context
+    sets are compared with the SHA-256 prefixes recorded from the reference (tests/golden/reference_tables.json); the
+    matrices, state tables and scan orders are then pinned only through the end-to-end goldens."""
+    orc = R.oracle()
     if not os.path.exists(R.REF_SO):
-        pytest.skip("oracle/_ref not built")
-    ref, orc = R.ref(), R.oracle()
+        want = json.load(open(os.path.join(G.GOLD, "reference_tables.json")))["context_set_sha256_12"]
+        for q in range(5):
+            mine = (ctypes.c_ubyte * 142)()
+            orc.oracle_ctx_init(mine, q)
+            assert R.sha(bytes(mine))[:12] == want[q], q
+        return
+    ref = R.ref()
     for t, (sym, n) in enumerate([("DST4_MAT", 4), ("DCT8_MAT", 8), ("DCT16_MAT", 16), ("DCT32_MAT", 32)]):
         m = np.ctypeslib.as_array((ctypes.c_int * (n * 32)).in_dll(ref, sym)).reshape(n, 32)[:, :n]
         mine = np.array([[orc.oracle_tm(t, k, i) for i in range(n)] for k in range(n)])
@@ -89,9 +98,18 @@ def test_generated_tables_match_reference_exports():
 
 
 def test_header_bytes_match_reference():
+    """The oracle's header bytes against the reference's putHeaderToBuffer; where oracle/_ref is absent, against the
+    first bytes of every stream the reference wrote for the small goldens (five padded sizes x qpd6 0..4)."""
+    orc = R.oracle()
     if not os.path.exists(R.REF_SO):
-        pytest.skip("oracle/_ref not built")
-    ref, orc = R.ref(), R.oracle()
+        data, _ = G.small_cases()
+        for name in G.small_case_names():
+            for q in range(5):
+                b = (ctypes.c_ubyte * 256)()
+                nb = orc.oracle_header(b, q, *data[f"{name}/q{q}/rcon"].shape)
+                assert bytes(b[:nb]) == data[f"{name}/q{q}/stream"].tobytes()[:nb], (name, q)
+        return
+    ref = R.ref()
     for q in range(5):
         for (h, w) in ((32, 32), (512, 768), (768, 512), (2176, 3840), (8192, 8192), (64, 96)):
             a = (ctypes.c_ubyte * 256)()

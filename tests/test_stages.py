@@ -28,9 +28,7 @@ class Cab(ctypes.Structure):
 
 
 @pytest.fixture(scope="module")
-def libs():
-    if not os.path.exists(R.REF_SO):
-        pytest.skip("oracle/_ref not built (needs the reference tree)")
+def ours():
     srcs = [os.path.join(S.SIM_DIR, "hevce_simstage.cpp"), os.path.join(S.CSRC, "hevce_core.h")]
     if not os.path.exists(STAGE_SO) or any(os.path.getmtime(STAGE_SO) < os.path.getmtime(s) for s in srcs):
         subprocess.run(["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-I", S.CSRC, "-o", STAGE_SO, srcs[0]], check=True)
@@ -42,6 +40,13 @@ def libs():
     if not os.path.exists(plain_so) or any(os.path.getmtime(plain_so) < os.path.getmtime(x) for x in srcs):
         subprocess.run(["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-DHEVCE_OPT_BYPMERGE=0", "-I", S.CSRC, "-o", plain_so, srcs[0]], check=True)
     ours.plain = ctypes.CDLL(plain_so)
+    return ours
+
+
+@pytest.fixture(scope="module")
+def libs(ours):
+    if not os.path.exists(R.REF_SO):
+        pytest.skip("oracle/_ref not built (needs the reference tree)")
     ref = ctypes.CDLL(R.REF_SO, mode=ctypes.RTLD_LOCAL)
     ref.newContextSet.restype = Ctx
     ref.newContextSet.argtypes = [ctypes.c_int]
@@ -148,6 +153,16 @@ def test_rdoq_every_coefficient_value(libs, T):
         assert len(bad) == 0, (T, q, int(vals[bad[0]]), int(got[bad[0]]), int(want[bad[0]]))
 
 
+def test_probability_state_63_is_unreachable(ours):
+    """Probability state 63 (context bytes 126, 127) is closed off in the kernel's tables: no transition from a lower
+    state and no initial value of any context reaches it, so the renormalisation shift computed from the LPS range
+    never meets the one state where it differs from the reference's table."""
+    st, dr, cx = (ctypes.c_int * (128 * 6))(), (ctypes.c_int * 8)(), (ctypes.c_int * (5 * 92))()
+    assert ours.hevce_stage_tables(st, dr, cx) == 92
+    assert all(st[v * 6 + 4] < 126 and st[v * 6 + 5] < 126 for v in range(126))
+    assert all(cx[i] < 126 for i in range(5 * 92))
+
+
 def test_coder_tables_match_the_reference_tables(libs):
     """The kernel's packed tables against the arrays and functions the reference exports: the 64-bit word per context
     state (LPS ranges, both next states: CABAC_LPS_TABLE, CONTEXT_NEXT_STATE_LPS / _MPS, HEVCe.c:701-713), the
@@ -168,9 +183,6 @@ def test_coder_tables_match_the_reference_tables(libs):
             if v < 126:   # probability state 63 is reserved for the terminate bin (no context ever holds it)
                 assert 9 - r.bit_length() == renorm[r >> 3], (v, q, r)
         assert (st[v * 6 + 4], st[v * 6 + 5]) == (nlps[v], nmps[v]), v
-    # probability state 63 (context bytes 126, 127) is closed off: no transition from a lower state and no initial value reaches it
-    assert all(st[v * 6 + 4] < 126 and st[v * 6 + 5] < 126 for v in range(126))
-    assert all(cx[i] < 126 for i in range(5 * 92))
     ref.estimateCoeffRate.restype = ctypes.c_int
     rate = [ref.estimateCoeffRate(l) for l in range(0, 9000)]
     for l in range(1, 9000):      # levels reach 8192 (|coefficient| <= 32767 at qpd6 = 0, 32x32)
@@ -214,19 +226,28 @@ def our_residual(ours, T, mode, q, lev):
     return bits, tuple(st)
 
 
-def test_residual_coding_spot_values(libs):
-    """The known answers of SURVEY.md section 8c (fresh coder, fresh contexts)."""
-    ours, ref = libs
+def spot_blocks():
     z = np.zeros((4, 4), np.int32)
-    assert our_residual(ours, 4, 0, 2, z)[0] == 4                      # putCoef on an all-zero block codes last=(0,0)
     a = z.copy(); a[0, 0] = 5; a[1, 2] = -1
-    bits, st = our_residual(ours, 4, 26, 2, a)
-    assert bits == 25 and st[:5] == (464, 126432, 14, 1, 191) and st[6] == 1
     b = np.zeros((8, 8), np.int32); b[0, 0] = -12; b[3, 3] = 2; b[7, 7] = 1
-    assert our_residual(ours, 8, 10, 0, b)[0] == 52
     c = np.zeros((32, 32), np.int32); c[0, 0] = 300; c[31, 31] = -1
-    assert our_residual(ours, 32, 1, 4, c)[0] == 61
-    for T, m, q, blk in ((4, 0, 2, z), (4, 26, 2, a), (8, 10, 0, b), (32, 1, 4, c)):
+    return ((4, 0, 2, z), (4, 26, 2, a), (8, 10, 0, b), (32, 1, 4, c))
+
+
+def test_residual_coding_spot_values(ours):
+    """The known answers of SURVEY.md section 8c (fresh coder, fresh contexts), measured on the reference."""
+    z, a, b, c = spot_blocks()
+    assert our_residual(ours, *z)[0] == 4                              # putCoef on an all-zero block codes last=(0,0)
+    bits, st = our_residual(ours, *a)
+    assert bits == 25 and st[:5] == (464, 126432, 14, 1, 191) and st[6] == 1
+    assert our_residual(ours, *b)[0] == 52
+    assert our_residual(ours, *c)[0] == 61
+
+
+def test_residual_coding_spot_values_match_putcoef(libs):
+    """The same blocks, every field of the call-for-call build's coder state against the reference's putCoef."""
+    ours, ref = libs
+    for T, m, q, blk in spot_blocks():
         assert our_residual(ours.plain, T, m, q, blk) == ref_residual(ref, T, m, q, blk)
 
 
@@ -262,12 +283,11 @@ def test_residual_coding_matches_putcoef(libs, T):
         assert st[3] + st[6] == want[1][3] + want[1][6], (T, mode, q, kind, trial)               # bytes produced (pending + written)
 
 
-def test_bypass_grouping_does_not_change_the_bytes(libs):
+def test_bypass_grouping_does_not_change_the_bytes(ours):
     """The kernel codes the bypass strings of one syntax element with one call where the reference issues several (one
     per bit for the last-position suffixes, prefix and suffix of an escape level separately).  Bypass coding is linear
     and bytes leave the coder's window at the same bit positions whatever the grouping: 300 random sequences of context
     bins and bypass strings (incl. zero runs that trigger emulation prevention) give identical byte streams."""
-    ours, _ = libs
     n = ctypes.c_int(0)
     total = 0
     for seed in range(300):
