@@ -2,7 +2,7 @@
 // (reference samples, 35 predictors, integer transforms, simplified RDOQ, reconstruction, CABAC trial coding,
 // CU quadtree decision, bitstream commit) as code for ONE CTA that encodes ONE picture.
 //
-// The file is compiled by nvcc into the sm_100a kernel (hevce_kernel.cu).  It contains no CPU fallback: the
+// The file is compiled by nvcc into the sm_100a kernel (hevce_variant.cu).  It contains no CPU fallback: the
 // product library only ever runs it on the GPU.  For development the same source is also compiled by g++ into a
 // single-threaded *simulator* of the CTA (tests/sim/, test infrastructure only), where every PAR_FOR phase runs
 // its work items in a permuted order; bit-exactness under permutation shows the phases are race-free.
@@ -33,22 +33,7 @@
 #define HEVCE_NOINLINE __attribute__((noinline))
 #endif
 
-// tuning switches: tools/ab_variants.py builds A/B variants of the library with -DHEVCE_OPT_xxx=0/1
-// measured on B200 (tools/ab_variants.py, 888 x 64x64, qpd6=2): LPS4=1 +1.5 %, FLUSH=1 +4 % kernel time -> both off;
-// BINSEL neutral; GANG 6 (80 regs) = GANG 5 (96 regs) > GANG 4 by 12 %; GANG 7 (72 regs, possible since the context
-// sets shrank to 26 words) 5.7 % more pictures per second per SM than GANG 6.
-#ifndef HEVCE_OPT_LPS4
-#define HEVCE_OPT_LPS4 0
-#endif
-#ifndef HEVCE_OPT_FLUSH
-#define HEVCE_OPT_FLUSH 0
-#endif
-#ifndef HEVCE_OPT_PREFETCH   // next coefficient group: 0 none, 1 register double buffer, 2 prefetch.global.L1 (measured: 47.0 / 47.5 / 46.95 ms)
-#define HEVCE_OPT_PREFETCH 2
-#endif
-#ifndef HEVCE_OPT_BINSEL
-#define HEVCE_OPT_BINSEL 1
-#endif
+// tuning switches: tools/ab_variants.py builds A/B variants of the library with other values of them
 // Consecutive bypass strings of one syntax element coded by ONE put_bypass call (the reference issues one call per bit of
 // the last-position suffixes and two per escape level, HEVCe.c:1076-1086, 1154-1169).  Exact for everything observable:
 // bypass coding is linear (low = low * 2^n + range * bits) and a byte leaves the window whenever fewer than 12 bits of
@@ -60,32 +45,6 @@
 #ifndef HEVCE_OPT_BYPMERGE
 #define HEVCE_OPT_BYPMERGE 1
 #endif
-// Trial coder: the common byte release (exactly one pending byte, its value above 3, so no emulation-prevention byte and
-// no zero run can be involved) as a short straight path in front of the general state machine.
-#ifndef HEVCE_OPT_FASTREL
-#define HEVCE_OPT_FASTREL 0
-#endif
-// put_bin: one 32-bit table word per (context state, range quarter) carrying the LPS range, the LPS renormalisation
-// shift and both next states (one shared-memory load per bin instead of two or three plus the shift arithmetic)
-// 1: word per (state, range quarter), plain load; 2: the same through an explicit ld.shared (no re-derived window base);
-// 3: one 64-bit word per state (the four LPS ranges + both next states) loaded as soon as the context byte is known: the
-//    load no longer waits for the previous bin's range, which leaves the range recurrence shift -> byte select -> subtract ->
-//    compare -> select -> shift, all register arithmetic
-#ifndef HEVCE_OPT_BINTAB
-#define HEVCE_OPT_BINTAB 3
-#endif
-// consecutive bins of a loop that hit the same context take its state from a register instead of reading back the byte
-// they have just stored
-#ifndef HEVCE_OPT_CTXFWD
-#define HEVCE_OPT_CTXFWD 0
-#endif
-// Trial coder, byte release: the common case (exactly one pending byte, the new lead byte is not 0xFF, the released byte is
-// above 3 so neither an emulation-prevention byte nor a zero run is involved) as predicated straight-line code on every
-// bin; only the rare cases branch.  With 32 lanes per warp some lane releases a byte on nearly every bin, so the branchy
-// version is paid in full almost every time.
-#ifndef HEVCE_OPT_RELPRED
-#define HEVCE_OPT_RELPRED 0
-#endif
 // bit-fields of a coefficient group built two levels at a time (signs gathered by shift + mask, the non-zero mask squeezed
 // out of the class field) instead of level by level: 100 instead of 159 instructions per group.  Measured (profiles/
 // r2_ab_fastbuild_*.log): -0.7 % on the one-picture-per-CTA cluster variant, +0.6 % on the 7-picture gang, where the longer
@@ -93,13 +52,11 @@
 #ifndef HEVCE_OPT_FASTBUILD
 #define HEVCE_OPT_FASTBUILD (HEVCE_OPT_GANG == 1)
 #endif
-// RDOQ evaluates the two candidate levels that can win (proof at phase_b_item); 0 = all three of HEVCe.c:571
-#ifndef HEVCE_OPT_RDOQ2
-#define HEVCE_OPT_RDOQ2 1
-#endif
 // ---- kernel variant (one translation unit per variant, see hevce_variant.cu): pictures per CTA, threads per picture,
 // trial lanes per warp and the pool plan.  GANG x NT threads run in lock-step phases; WIDE = one picture owns the CTA
-// and most of the SM's shared memory (all 35 candidates of a 16x16 / 32x32 step in one round).
+// and most of the SM's shared memory (all 35 candidates of a 16x16 / 32x32 step in one round).  Measured on B200
+// (888 x 64x64, qpd6=2): GANG 6 (80 regs) = GANG 5 (96 regs) > GANG 4 by 12 %; GANG 7 (72 regs, possible since the
+// context sets shrank to 26 words) 5.7 % more pictures per second per SM than GANG 6.
 #ifndef HEVCE_OPT_GANG
 #define HEVCE_OPT_GANG 7
 #endif
@@ -169,7 +126,6 @@ constexpr int CTXW = 23;           // context words per lane (odd: lane-major co
 constexpr int CTXW4 = 9;           // leading words that hold every context a 4x4 luma TU's residual can touch
 constexpr int WP = 65;             // pitch of the CTU reconstruction window (row 0 / col 0 = neighbours)
 constexpr int IMAX = 0x7fffffff;
-constexpr int LANE_ELEMS = CTU * CTU;
 
 // Compact layout (the reference struct also carries the chroma contexts, 142 bytes).  What the residual of a 4x4 luma TU
 // touches comes first, so an NxN PU lane initialises words 0..CTXW4-1 only: last_x of 4x4 TUs 0-2, last_y of 4x4 TUs 3-5,
@@ -201,6 +157,8 @@ HEVCE_HD inline int bitlen(unsigned v) {
 // ------------------------------------------------------------------------------------------------------------
 // constant tables (filled on the host by fill_tables(), copied to __constant__ and from there to shared memory)
 // ------------------------------------------------------------------------------------------------------------
+// bin4, sigp4 and rate32 have no reader, and lps4 / next_lps only feed st8.  They stay: dropping them moves the other
+// fields, and that layout measured 0.2-0.6 % slower on the gang variants (profiles/r2_notes.md).
 struct Tables {
     u32 lps4[64];          // rangeTabLps, one word per state: byte q = LPS range for (range>>6)&3 == q  (HEVCe.c:704-713)
     u8 next_lps[128];      // (state<<1|mps) after an LPS                   (HEVCe.c:702)
@@ -350,13 +308,13 @@ struct BacT {
     Coder c;
     u8* out;            // EMIT only: destination of this CTU's bytes
     int cap;            // EMIT only: bytes available at out
-    u32 tabs;           // device: shared-space address of Tables::bin4, kept in a register (use_tables)
+    u32 tabs;           // device: shared-space address of Tables::st8, kept in a register (use_tables)
 
     // The bin table is read with an explicit ld.shared from an address the compiler cannot re-derive: left to itself it
     // rebuilds the shared-window base (S2UR + UMOV + ULEA) in front of every bin.
     HEVCE_HD void use_tables(const Tables& tb) {
-#if defined(__CUDA_ARCH__) && HEVCE_OPT_BINTAB >= 2
-        tabs = HEVCE_OPT_BINTAB == 2 ? (u32)__cvta_generic_to_shared(&tb.bin4[0]) : (u32)__cvta_generic_to_shared(&tb.st8[0]);
+#if defined(__CUDA_ARCH__)
+        tabs = (u32)__cvta_generic_to_shared(&tb.st8[0]);
         asm volatile("mov.u32 %0, %0;" : "+r"(tabs));
 #else
         (void)tb; tabs = 0;
@@ -381,67 +339,21 @@ struct BacT {
         }
     }
     HEVCE_HD void carry_out() {   // HEVCe.c:859-879
-#if HEVCE_OPT_RELPRED
-        if (!EMIT) {
-            const bool rel = c.nbits < 12;
-            const int lead9 = c.low >> (24 - c.nbits);               // meaningful when rel (the shift count stays in 1..24 anyway)
-            const int b9 = (c.held + (lead9 >> 8)) & 0xff;
-            const bool common = (lead9 != 0xff) & (c.nbytes == 1) & (b9 > 3);
-            if (rel & common) {
-                c.nbits += 8;
-                c.low &= (int)(0xFFFFFFFFu >> c.nbits);
-                c.n += 1;
-                c.z = 0;
-                c.held = lead9 & 0xff;
-                return;
-            }
-            if (!rel) return;
-        }
-#endif
         if (c.nbits >= 12) return;
         const int lead = c.low >> (24 - c.nbits);
         c.nbits += 8;
         c.low &= (int)(0xFFFFFFFFu >> c.nbits);
-#if HEVCE_OPT_FASTREL
-        if (!EMIT) {
-            const int b = (c.held + (lead >> 8)) & 0xff;
-            if (lead != 0xff && (c.nbytes == 0 || (c.nbytes == 1 && b > 3))) {
-                c.n += c.nbytes;
-                c.z = c.nbytes ? 0 : c.z;
-                c.held = c.nbytes ? (lead & 0xff) : lead;
-                c.nbytes = 1;
-                return;
-            }
-        }
-#endif
-        if (EMIT || !HEVCE_OPT_FLUSH) {
-            if (lead == 0xff) c.nbytes++;
-            else if (c.nbytes > 0) {
-                const int carry = lead >> 8;
-                emit(c.held + carry);
-                c.held = lead & 0xff;
-                for (; c.nbytes > 1; c.nbytes--) emit((0xff + carry) & 0xff);
-            } else { c.nbytes = 1; c.held = lead; }
-        } else {
-            // Trial coder: the same state machine with the common case (release the held byte) branch-free.  In a warp
-            // some lane takes this path on most bins, so its length is paid almost every time.
-            const int ff = lead == 0xff, had = c.nbytes > 0, rel = !ff & had, carry = lead >> 8;
-            const int b = (c.held + carry) & 0xff;
-            const int epb = rel & (c.z >= 2) & (b <= 3);
-            c.n += rel + epb;
-            c.z = rel ? (b ? 0 : (epb ? 1 : c.z + 1)) : c.z;
-            if (rel & (c.nbytes > 1)) {   // rare: a run of pending 0xFF bytes is released behind it
-                for (; c.nbytes > 1; c.nbytes--) emit((0xff + carry) & 0xff);
-            }
-            c.held = ff ? c.held : (had ? (lead & 0xff) : lead);
-            c.nbytes = ff ? c.nbytes + 1 : 1;
-        }
+        if (lead == 0xff) c.nbytes++;
+        else if (c.nbytes > 0) {
+            const int carry = lead >> 8;
+            emit(c.held + carry);
+            c.held = lead & 0xff;
+            for (; c.nbytes > 1; c.nbytes--) emit((0xff + carry) & 0xff);
+        } else { c.nbytes = 1; c.held = lead; }
     }
     HEVCE_HD void put_bin(const Tables& tb, int bin, u8& cx) { cx = (u8)bin_step(tb, bin, cx); }
     // one context-coded bin with context byte v; returns the new context byte (HEVCe.c:914-933, both branches computed, then selected)
     HEVCE_HD int bin_step(const Tables& tb, int bin, const int v) {
-        int cxn;
-#if HEVCE_OPT_BINTAB == 3
 #if defined(__CUDA_ARCH__)
         u32 lo, hi;
         asm("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(lo), "=r"(hi) : "r"(tabs + (u32)v * 8u));
@@ -463,65 +375,9 @@ struct BacT {
         c.low = (int)((unsigned)c.low << sh);
         c.range = (is_lps ? lps : rmps) << sh;
         c.nbits -= sh;
-        cxn = (int)((is_lps ? hi : hi >> 8) & 0xffu);
+        const int cxn = (int)((is_lps ? hi : hi >> 8) & 0xffu);
 #if !defined(__CUDA_ARCH__)
         if (v >= 126 || (unsigned)bin > 1u || c.range < 256 || c.range > 510) __builtin_trap();
-#endif
-#elif HEVCE_OPT_BINTAB
-#if defined(__CUDA_ARCH__) && HEVCE_OPT_BINTAB == 2
-        u32 w;
-        asm("ld.shared.u32 %0, [%1];" : "=r"(w) : "r"(tabs + (u32)(v * 4 + (c.range >> 6)) * 4u));
-#else
-        const u32 w = tb.bin4[v * 4 + (c.range >> 6)];              // 256 <= range <= 510 between bins
-#endif
-        const int lps = (int)(w & 0xffu);
-        const int rmps = c.range - lps;
-        const bool is_lps = ((v ^ bin) & 1) != 0;                   // bin is 0 or 1 at every call site
-        const int sh = is_lps ? (int)(w >> 29) : (rmps < 256 ? 1 : 0);
-        if (is_lps) c.low += rmps;
-        c.low = (int)((unsigned)c.low << sh);
-        c.range = (is_lps ? lps : rmps) << sh;
-        c.nbits -= sh;
-        u32 nx = w >> 8;
-        if (!is_lps) nx >>= 8;
-        cxn = (int)(nx & 0xffu);
-#if !defined(__CUDA_ARCH__)
-        if ((unsigned)bin > 1u || c.range < 256 || c.range > 510) __builtin_trap();
-#endif
-#else
-#if HEVCE_OPT_LPS4
-        const int lps = (int)((tb.lps4[v >> 1] >> (((c.range >> 6) & 3) * 8)) & 0xffu);   // the load depends on the context only, not on range
-#else
-        const int lps = ((const u8*)tb.lps4)[(v >> 1) * 4 + ((c.range >> 6) & 3)];
-#endif
-#if HEVCE_OPT_BINSEL
-        const int nlps = tb.next_lps[v];
-        const int rmps = c.range - lps;
-        const bool is_lps = ((v ^ bin) & 1) != 0;                   // bin is 0 or 1 at every call site
-        // renorm table, HEVCe.c:715: 9 - bitlen(lps) for lps >= 6; the only smaller entry (2, probability state 63) cannot
-        // be reached: contexts are initialised to states 1..126 (ctx_init_value) and the MPS transition stops at 62
-        const int nb = 9 - bitlen((unsigned)lps);
-#if !defined(__CUDA_ARCH__)
-        if (v >= 126 || (unsigned)bin > 1u) __builtin_trap();
-#endif
-        const int sh = is_lps ? nb : (rmps < 256 ? 1 : 0);
-        c.low = (int)((unsigned)(is_lps ? c.low + rmps : c.low) << sh);
-        c.range = (is_lps ? lps : rmps) << sh;
-        c.nbits -= sh;
-        cxn = is_lps ? nlps : (v < 124 ? v + 2 : v);                // HEVCe.c:701-702
-#else
-        c.range -= lps;
-        if ((bin != 0) != ((v & 1) != 0)) {
-            const int nb = lps < 8 ? 6 : 9 - bitlen((unsigned)lps);
-            cxn = tb.next_lps[v];
-            c.low = (int)((unsigned)(c.low + c.range) << nb);
-            c.range = lps << nb;
-            c.nbits -= nb;
-        } else {
-            cxn = v < 124 ? v + 2 : v;
-            if (c.range < 256) { c.low = (int)((unsigned)c.low << 1); c.range <<= 1; c.nbits--; }
-        }
-#endif
 #endif
         carry_out();
         return cxn;
@@ -1047,42 +903,11 @@ HEVCE_HD inline void code_group(BAC& b, const Tables& tbl, const Cx cx, int s, i
         const bool dc = first_cg && s != 4;                         // position 0 of a larger TU has its own context
         int k = is_last ? kstart - 1 : 15;
         const int kend = (!first_cg && (nzm & ~1u) == 0) ? 1 : 0;   // position 0 of a later group is inferred when it is the only one
-#if HEVCE_OPT_CTXFWD == 2
-        // software pipeline: the context byte of the next bin is loaded before the arithmetic of this one; when both bins
-        // share the context, the state comes from the register instead
-        if (k >= kend) {
-            auto ctx_of = [&](int kk) -> int { const int c0 = base + (int)((tab >> (4 * kk)) & 15u); return (dc && kk == 0) ? (int)CX_SIG : c0; };
-            int ci = ctx_of(k), v = cx[ci];
-            for (;;) {
-                const bool more = k > kend;
-                int cin = ci, vn = 0;
-                if (more) { cin = ctx_of(k - 1); vn = cx[cin]; }
-                const int nv = b.bin_step(tbl, (int)((nzm >> k) & 1u), v);
-                cx[ci] = (u8)nv;
-                if (!more) break;
-                v = cin == ci ? nv : vn;
-                ci = cin;
-                k--;
-            }
-        }
-#else
-#if HEVCE_OPT_CTXFWD
-        int pci = -1, pv = 0;
-#endif
         for (; k >= kend; k--) {
             int ci = base + (int)((tab >> (4 * k)) & 15u);
             if (dc && k == 0) ci = CX_SIG;
-#if HEVCE_OPT_CTXFWD
-            int v = cx[ci];
-            if (ci == pci) v = pv;
-            pv = b.bin_step(tbl, (int)((nzm >> k) & 1u), v);
-            cx[ci] = (u8)pv;
-            pci = ci;
-#else
             b.put_bin(tbl, (int)((nzm >> k) & 1u), cx[ci]);
-#endif
         }
-#endif
     }
     if (nzm) {
         // ---- greater1 / greater2 flags, signs (HEVCe.c:1229-1252)
@@ -1090,24 +915,13 @@ HEVCE_HD inline void code_group(BAC& b, const Tables& tbl, const Cx cx, int s, i
         int nz = 0, signs = 0, g2 = -1;
         c1 = 1;
         unsigned mm = nzm;
-#if HEVCE_OPT_CTXFWD == 1
-        int pc1 = -1, pv1 = 0;
-#endif
         while (mm) {
             const int k = bitlen(mm) - 1;
             mm &= ~(1u << k);
             signs = (signs << 1) | (int)((sgn >> k) & 1u);
             if (nz < 8) {
                 const int a = (int)((cls >> (2 * k)) & 3u), big = a > 1;
-#if HEVCE_OPT_CTXFWD == 1
-                int v1 = cx[CX_ONE + 4 * set + c1];
-                if (c1 == pc1) v1 = pv1;
-                pv1 = b.bin_step(tbl, big, v1);
-                cx[CX_ONE + 4 * set + c1] = (u8)pv1;
-                pc1 = c1;
-#else
                 b.put_bin(tbl, big, cx[CX_ONE + 4 * set + c1]);
-#endif
                 if (big) { c1 = 0; if (g2 < 0) g2 = a > 2; else g2 |= 4; }
                 else if (c1 > 0 && c1 < 3) c1++;
             }
@@ -1189,9 +1003,6 @@ HEVCE_HD inline void put_residual(BAC& b, const Tables& tbl, const Cx cx, int s,
     // groups are visited in reverse scan order; the levels of the next coded group are fetched while the current
     // one is being coded (the store is L2-resident, a fetch costs several hundred cycles)
     u32 w[8];
-#if HEVCE_OPT_PREFETCH == 1
-    u32 wn[8];
-#endif
     int cy, cxg, ncy = 0, ncx = 0;
     cgpos(gl, cy, cxg);
     int on = bit(cy, cxg);
@@ -1204,9 +1015,7 @@ HEVCE_HD inline void put_residual(BAC& b, const Tables& tbl, const Cx cx, int s,
             if (bit(ncy, ncx)) { on2 = 1; break; }
         }
         if (g2 == 0) { ncy = 0; ncx = 0; on2 = g > 0 ? bit(0, 0) : 0; }
-#if HEVCE_OPT_PREFETCH == 1
-        if (on2) load_group(lev + (ncy * ncg + ncx) * 16, wn);
-#elif HEVCE_OPT_PREFETCH == 2 && defined(__CUDA_ARCH__)
+#if defined(__CUDA_ARCH__)
         if (on2) asm volatile("prefetch.global.L1 [%0];" ::"l"(lev + (ncy * ncg + ncx) * 16));
 #endif
         const int first_cg = g == 0;
@@ -1224,12 +1033,7 @@ HEVCE_HD inline void put_residual(BAC& b, const Tables& tbl, const Cx cx, int s,
             b.put_bin(tbl, 0, cx[CX_SIGCG + ((rgt | dwn) != 0)]);
         }
         g = g2; cy = ncy; cxg = ncx; on = on2;
-#if HEVCE_OPT_PREFETCH == 1
-#pragma unroll
-        for (int i = 0; i < 8; i++) w[i] = wn[i];
-#else
         if (on) load_group(lev + (cy * ncg + cxg) * 16, w);
-#endif
     }
 }
 
@@ -1329,13 +1133,6 @@ HEVCE_HD inline void scan_groups(const s16* lev, int s, unsigned& mlo, unsigned&
             load_group(lev + (gy * ncg + gx) * 16, w);
             if (w[0] | w[1] | w[2] | w[3] | w[4] | w[5] | w[6] | w[7]) { const int k = gy * 8 + gx; if (k < 32) mlo |= 1u << k; else mhi |= 1u << (k - 32); }
         }
-}
-
-
-// trial lanes: thread -> candidate, packed into as few warps as possible.  (Spreading the 70 lanes evenly over the
-// four warps was measured 12 % slower: the trial phase is issue-bound, a warp instruction costs the same with 18 lanes.)
-HEVCE_HD inline int lane_to_cand(int n, int t) {   // returns the candidate index < n, or -1
-    return t < n ? t : -1;
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -1510,7 +1307,6 @@ HEVCE_HD inline int rdoq_level(int cf, const RdoqK& k, const Tables& tb, int& dl
     dl = iabs(cf) << 14;                                         // |cf| <= 32767: the clamps of HEVCe.c:566 cannot trigger
     const int lvl = (dl + k.add) >> k.sh;
     if (lvl <= 0) return 0;
-#if HEVCE_OPT_RDOQ2
     // Candidates lvl and lvl-1 only: the third one of HEVCe.c:571, lvl-2, can never be picked.  One level is
     // U = 2^(11+q) in units of the distance e; e(lvl) <= U/2, e(lvl-1) = a in [U/2, 3U/2), e(lvl-2) = a + U exactly
     // (2^sh is a multiple of 2^dsh).  qpd6 <= 3: nothing saturates (5U/2 < 46340) and dist(lvl-2) - dist(lvl-1) >=
@@ -1529,20 +1325,6 @@ HEVCE_HD inline int rdoq_level(int cf, const RdoqK& k, const Tables& tb, int& dl
     const int d1 = (e1 < 46340 ? e1 * e1 : IMAX) >> 7;          // saturates at qpd6 = 4 only
     const int dr = tb.drate[imin(lvl, 7)] + ((lvl >= 7 && ((lvl - 5) & (lvl - 6)) == 0) ? 65536 : 0);
     return k.wd * (d1 - d0) < k.wb * dr ? lvl - 1 : lvl;
-#else
-    // candidates lvl, lvl-1, lvl-2 (>= 0); strict '<' scanning downwards: the highest level wins ties
-    int pick = lvl, best = IMAX;
-#pragma unroll
-    for (int t = 0; t < 3; t++) {
-        const int l = lvl - t;
-        const int d1 = iabs(dl - (l << k.sh)) >> k.dsh;
-        const int d = (d1 < 46340 ? d1 * d1 : IMAX) >> 7;
-        const int wr = k.wb * (l < 32 ? tb.rate32[imax(l, 0)] : 92000 + ((4 + 2 * (bitlen((unsigned)(l - 5)) - 1)) << 15));   // HEVCe.c:526-535
-        const int cost = k.wd * d + wr;
-        if (l >= 0 && cost < best) { best = cost; pick = l; }
-    }
-    return pick;
-#endif
 }
 
 // phase B: forward row transform (HEVCe.c:515) + per-coefficient RDOQ (HEVCe.c:563-586); tentative levels replace

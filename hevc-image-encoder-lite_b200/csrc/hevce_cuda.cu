@@ -1,7 +1,8 @@
 // hevce_cuda.cu -- sm_100a kernels + device-resident sessions of libhevce_b200.so.
 //
 // The decision kernel (hevce_core.h: encode_picture) is linked in several variants (hevce_variant.cu, hevce_variants.h):
-// gangs of 7 / 4 / 2 pictures per CTA and one "wide" picture per CTA.  This file picks the variant per batch, owns the
+// gangs of 7 / 4 / 2 pictures per CTA, one "wide" picture per CTA, and one picture per CTA or per cluster of two CTAs
+// split into parent || child tracks.  This file picks the variant per batch, owns the
 // commit / quality / peak kernels and everything between the plain-C API (hevce_api.c) and the device.
 //
 // Host side here is the thin layer between the plain-C API (hevce_api.c) and the device: buffer management in HBM,
@@ -114,12 +115,12 @@ struct Variant {
     void (*info)(hevce_variant_info*);
     void (*profile)(unsigned long long*, unsigned long long*);
     hevce_variant_info vi;
-    double cost;   // relative time per CTU of one gang when the whole GPU runs this variant (measured, see DESIGN.md)
+    double cost;   // relative time per CTU of one gang when the whole GPU runs this variant (HEVCE_VARIANT_LIST)
 };
 #if defined(HEVCE_PROFILE_DUMP)
-#define HEVCE_VARIANT_ROW(tag, g, nt, lpw, wide) {#tag, hevce_variant_prepare_##tag, hevce_variant_launch_##tag, hevce_variant_info_##tag, hevce_variant_profile_##tag, {}, 0.0},
+#define HEVCE_VARIANT_ROW(tag, cost) {#tag, hevce_variant_prepare_##tag, hevce_variant_launch_##tag, hevce_variant_info_##tag, hevce_variant_profile_##tag, {}, cost},
 #else
-#define HEVCE_VARIANT_ROW(tag, g, nt, lpw, wide) {#tag, hevce_variant_prepare_##tag, hevce_variant_launch_##tag, hevce_variant_info_##tag, nullptr, {}, 0.0},
+#define HEVCE_VARIANT_ROW(tag, cost) {#tag, hevce_variant_prepare_##tag, hevce_variant_launch_##tag, hevce_variant_info_##tag, nullptr, {}, cost},
 #endif
 Variant g_variants[] = {HEVCE_VARIANT_LIST(HEVCE_VARIANT_ROW)};
 constexpr int NVARIANT = (int)(sizeof(g_variants) / sizeof(g_variants[0]));
@@ -131,9 +132,7 @@ std::once_flag g_variants_once;
 void variants_init() {
     std::call_once(g_variants_once, [] {
         fill_tables(g_host_tables);
-        // relative per-CTU latency of a gang (all SMs busy with the same variant), measured on B200 -- profiles/r2_notes.md
-        static const double kCost[NVARIANT] = {1.00, 0.74, 0.63, 0.54, 0.52, 0.30};   // 8.63 / 6.38 / 5.42 / 4.65 / 4.46 / 2.61 ms per CTU of one gang (148 gangs of 64x64 pictures, 74 for c2), qpd6=2
-        for (int v = 0; v < NVARIANT; v++) { g_variants[v].info(&g_variants[v].vi); g_variants[v].cost = kCost[v]; }
+        for (int v = 0; v < NVARIANT; v++) g_variants[v].info(&g_variants[v].vi);
         if (const char* env = getenv("HEVCE_VARIANT"))
             for (int v = 0; v < NVARIANT; v++) if (!strcmp(env, g_variants[v].name)) g_forced_variant = v;
     });
@@ -558,8 +557,8 @@ extern "C" int hevce_session_launches(const hevce_session* s) { return s ? s->la
 extern "C" int hevce_session_grid(const hevce_session* s) { return s ? s->grid : 0; }
 extern "C" const char* hevce_session_variant(const hevce_session* s) { return s ? g_variants[s->variant].name : ""; }
 
-// Kernel variant used for the batches configured from now on: "g7", "g4", "g2", "w1", or NULL / "" / "auto" to choose
-// per batch.  returns 0, or HEVCE_ERR_ARG for an unknown name.
+// Kernel variant used for the batches configured from now on: a tag of HEVCE_VARIANT_LIST, or NULL / "" / "auto" to
+// choose per batch.  returns 0, or HEVCE_ERR_ARG for an unknown name.
 extern "C" int hevce_set_variant(const char* name) {
     variants_init();
     if (!name || !*name || !strcmp(name, "auto")) { g_forced_variant = -1; return 0; }

@@ -12,19 +12,21 @@ typedef struct hevce_variant_info {
     long long smem_bytes;      /* dynamic shared memory per CTA                      */
 } hevce_variant_info;
 
-/* tag, pictures per CTA, threads per picture, lanes per warp, wide pool */
+/* tag, relative time per CTU of one gang when the whole GPU runs this variant: measured on B200 (qpd6=2, 148 gangs of
+ * 64x64 pictures, 74 for c2; profiles/r2_variant_latency.log, r2_variant_latency_c2.log), ms per CTU of one gang beside it.
+ * A variant's shape is set only by its VDEF_<tag> line in csrc/Makefile; hevce_variant_info_<tag>() reports it. */
 #define HEVCE_VARIANT_LIST(X) \
-    X(g7, 7, 128, 32, 0)      \
-    X(g4, 4, 224, 24, 0)      \
-    X(g2, 2, 448, 16, 0)       \
-    X(w1, 1, 896, 8, 1)       \
-    X(t1, 1, 896, 12, 0)      \
-    X(c2, 1, 896, 8, 0)
+    X(g7, 1.00) /* 8.63 */    \
+    X(g4, 0.74) /* 6.38 */    \
+    X(g2, 0.63) /* 5.42 */    \
+    X(w1, 0.54) /* 4.65 */    \
+    X(t1, 0.52) /* 4.46 */    \
+    X(c2, 0.30) /* 2.61 */
 
 #ifdef __cplusplus
 extern "C" {
 #endif
-#define HEVCE_DECLARE_VARIANT(tag, g, nt, lpw, wide)                                                                     \
+#define HEVCE_DECLARE_VARIANT(tag, cost)                                                                                 \
     int hevce_variant_prepare_##tag(void);                                                                               \
     int hevce_variant_launch_##tag(const void *jobs, const int *gangs, int ngangs, const void *slots, int *counter,      \
                                    const void *tables, int grid, void *stream);                                          \

@@ -163,7 +163,7 @@ def set_devices(ordinals):
 
 
 def set_variant(name=None):
-    """Kernel variant for the following batches: "g7", "g4", "g2", "w1", or None / "auto" to choose per batch."""
+    """Kernel variant for the following batches: "g7", "g4", "g2", "w1", "t1", "c2", or None / "auto" to choose per batch."""
     rc = lib().hevce_set_variant(name.encode() if name else None)
     if rc < 0:
         raise HevceError(rc, "hevce_set_variant")

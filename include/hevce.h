@@ -68,7 +68,7 @@ HEVCE_API int hevce_get_max_dim(void);   /* the limit in force; a call captures 
  * using stay.  The reference allocates nothing, so it has no counterpart. */
 HEVCE_API void hevce_release(void);
 
-/* Kernel variant for the batches configured from now on.  The decision kernel is linked in four variants of the same
+/* Kernel variant for the batches configured from now on.  The decision kernel is linked in six variants of the same
  * source: "g7" / "g4" / "g2" = 7 / 4 / 2 same-size pictures per CTA in lock-step (throughput), "w1" = one picture per
  * CTA with all its threads and nearly all shared memory of the SM, "t1" = one picture per CTA whose threads form three
  * tracks so that a 16x16 / 32x32 node's own candidates are evaluated while its children are decided, "c2" = the same

@@ -27,7 +27,7 @@ void sim_barrier(int id, int) { pthread_barrier_wait(&g_bar[id]); }
 extern "C" int hevce_simtrack_encode(unsigned char* out, int out_cap, const unsigned char* img, unsigned char* rcon,
                                      int* ysz, int* xsz, int q, int order, int* err) {
     using namespace HEVCE_NS;
-    static_assert(TRACKS, "compile with a parent || child variant (tests/simutil.py TRACK_FLAGS)");
+    static_assert(TRACKS, "compile with a parent || child variant (VDEF_t1 / VDEF_c2 in csrc/Makefile)");
     g_sim_order = order;
     static Tables tables;
     fill_tables(tables);

@@ -1,6 +1,7 @@
 """ctypes wrapper for the host-compiled kernel simulator (tests/sim, TEST INFRASTRUCTURE ONLY)."""
 import ctypes
 import os
+import re
 import subprocess
 
 import numpy as np
@@ -12,15 +13,22 @@ CSRC = os.path.join(ROOT, "hevc-image-encoder-lite_b200", "csrc")
 _u8p = ctypes.POINTER(ctypes.c_ubyte)
 
 
-# kernel variants (csrc/Makefile, hevce_variants.h): tag -> (pictures per CTA, threads per picture, lanes per warp, wide)
-VARIANTS = {"g7": (7, 128, 32, 0), "g4": (4, 224, 24, 0), "g2": (2, 448, 16, 0), "w1": (1, 896, 8, 1), "t1": (1, 896, 12, 0), "c2": (1, 896, 8, 0)}
-TRACK_FLAGS = {"t1": ["-DHEVCE_OPT_TRACKS=1", "-DHEVCE_OPT_TRK_C=448", "-DHEVCE_OPT_LPW_P=24"],       # parent || child variants
-               "c2": ["-DHEVCE_OPT_TRACKS=1", "-DHEVCE_OPT_CLUSTER=2", "-DHEVCE_OPT_LPW_P=8"]}
+def variants():
+    """The kernel variants linked into the library, {tag: compile flags}, from csrc/Makefile's VARIANTS and VDEF_<tag>
+    lines (the only place they are written)."""
+    mk = open(os.path.join(CSRC, "Makefile")).read()
+    line = lambda name: re.search(rf"^{name} := (.*)$", mk, re.M).group(1).split()
+    return {tag: line(f"VDEF_{tag}") for tag in line("VARIANTS")}
 
 
 def variant_flags(variant):
-    g, nt, lpw, wide = VARIANTS[variant]
-    return [f"-DHEVCE_OPT_GANG={g}", f"-DHEVCE_OPT_NT={nt}", f"-DHEVCE_OPT_LPW={lpw}", f"-DHEVCE_OPT_WIDE={wide}"] + TRACK_FLAGS.get(variant, [])
+    return variants()[variant]
+
+
+def variant_gang(variant):
+    """(pictures per CTA, CTAs per picture) of a variant."""
+    opt = dict(f.removeprefix("-DHEVCE_OPT_").split("=") for f in variant_flags(variant))
+    return int(opt["GANG"]), int(opt.get("CLUSTER", 0)) or 1
 
 
 def _build(src, so, variant, extra=()):

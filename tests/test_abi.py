@@ -60,6 +60,20 @@ def test_argument_validation_needs_no_gpu():
     assert (ys.value, xs.value) == (32, 32)
 
 
+def test_set_variant_accepts_every_makefile_variant():
+    """hevce_set_variant knows every kernel variant csrc/Makefile builds (HEVCE_VARIANT_LIST is in step with it) and
+    rejects any other tag.  No GPU needed: the variant table is filled by host-side functions only."""
+    import simutil as S
+    H = _ensure_built()
+    try:
+        for tag in S.variants():
+            H.set_variant(tag)
+        with pytest.raises(H.HevceError):
+            H.set_variant("g9")
+    finally:
+        H.set_variant(None)
+
+
 def test_no_cpu_fallback():
     """Without a CUDA device the product must fail loudly, never fall back to a CPU path."""
     try:

@@ -9,10 +9,11 @@ import pytest
 
 import golden_util as G
 import refutil as R
+import simutil as S
 import workloads as WL
 
 pytestmark = pytest.mark.gpu
-VARIANTS = ("g7", "g4", "g2", "w1", "t1", "c2")
+VARIANTS = tuple(S.variants())
 
 
 @pytest.fixture(scope="module")

@@ -5,20 +5,17 @@
 Each spec overrides -DHEVCE_OPT_<NAME>=<value> of the variant's flags in csrc/Makefile; the other variants are linked unchanged."""
 import glob
 import os
-import re
 import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CSRC = os.path.join(ROOT, "hevc-image-encoder-lite_b200", "csrc")
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+import simutil as S  # noqa: E402
+
 OUT = os.environ.get("HEVCE_AB_DIR") or os.path.join(ROOT, "hevc-image-encoder-lite_b200", "ab")
 ARCH = "-gencode arch=compute_100a,code=sm_100a"
 FLAGS = f"{ARCH} -O3 -lineinfo -std=c++17 -Xcompiler -fPIC,-fvisibility=hidden"
-
-
-def variant_defs(tag):
-    mk = open(os.path.join(CSRC, "Makefile")).read()
-    return re.search(rf"^VDEF_{tag} := (.*)$", mk, re.M).group(1).split()
 
 
 if sys.argv[1] == "build":
@@ -30,7 +27,7 @@ if sys.argv[1] == "build":
     others = [o for o in glob.glob(os.path.join(CSRC, "hevce_k_*.o")) if not o.endswith(f"hevce_k_{tag}.o")]
     procs = []
     for spec in ["base"] + specs:
-        defs = {d.split("=")[0]: d for d in variant_defs(tag)}
+        defs = {d.split("=")[0]: d for d in S.variant_flags(tag)}
         if spec != "base":
             for kv in spec.split(","):
                 k, v = kv.split("=")
@@ -47,10 +44,11 @@ else:
     tag = sys.argv[2]
     h, w, q = (sys.argv[3:6] + ["64", "64", "2"][len(sys.argv[3:6]):])
     code = ("import sys,os; sys.path.insert(0,'hevc-image-encoder-lite_b200'); sys.path.insert(0,'tests'); import numpy as np, hevce_b200 as H, workloads as WL;"
-            "H.LIB_PATH=sys.argv[1]; tag=sys.argv[2]; h,w,q=map(int,sys.argv[3:6]); g={'g7':7,'g4':4,'g2':2}.get(tag,1); n=148*g; K=WL.kodak_landscape();"
+            "H.LIB_PATH=sys.argv[1]; tag=sys.argv[2]; h,w,q,n=map(int,sys.argv[3:7]); K=WL.kodak_landscape();"
             "imgs=[WL.config3_image(i,K)[(37*i)%(512-h+1):,(53*i)%(768-w+1):][:h,:w].copy() for i in range(n)]; H.set_variant(tag);"
             "s=H.Session(0,[i.shape for i in imgs],q); s.upload(imgs); ms=[s.encode() for _ in range(4)]; st,_=s.download();"
             "import hashlib; print(os.path.basename(sys.argv[1]), ' '.join('%.2f'%m for m in ms), hashlib.sha256(b''.join(st)).hexdigest()[:12], flush=True)")
+    n = str(148 * S.variant_gang(tag)[0])   # a picture per CTA slot of 148 CTAs
     for rep in range(2):
         for so in sorted(glob.glob(os.path.join(OUT, "*.so"))):
-            subprocess.run([sys.executable, "-c", code, so, tag, h, w, q], cwd=ROOT)
+            subprocess.run([sys.executable, "-c", code, so, tag, h, w, q, n], cwd=ROOT)
