@@ -25,7 +25,8 @@
 #define POOL_PER_DEV 4                        /* cached sessions (grow-only buffers) per device ordinal */
 #define CHUNK_PIXELS (768LL * 1024 * 1024)    /* per-chunk bound (padded pixels) so the pinned staging stays modest */
 #define CHUNK_PICTURES 32768                  /* ... and pictures (the commit kernel's grid.y is the picture index) */
-#define WAVE_PICTURES (148 * 7)               /* pictures of one full wave of the 7-picture variant on a B200 */
+#define G7_GANG 7                             /* pictures per CTA of the g7 variant */
+#define WAVE_PICTURES (148 * G7_GANG)         /* pictures of one full wave of g7 on a B200 */
 #define MAX_WORKERS 4                         /* chunk workers per device (= cached sessions per device) */
 
 static pthread_mutex_t g_lock = PTHREAD_MUTEX_INITIALIZER;   /* device list + session pool */
@@ -37,7 +38,6 @@ static int g_pool_busy[MAX_DEV][POOL_PER_DEV];
 API const char *hevce_version(void) { return "hevce-b200 0.2 (sm_100a)"; }
 
 API int hevce_get_max_dim(void) { return __atomic_load_n(&g_max_dim, __ATOMIC_RELAXED); }
-int hevce_internal_max_dim(void) { return hevce_get_max_dim(); }
 
 API int hevce_set_max_dim(int max_dim) {
     int old = hevce_get_max_dim();
@@ -90,7 +90,7 @@ API int hevce_set_devices(int count, const int *ordinals) {
     return 0;
 }
 
-/* ---- session pool: concurrent callers (and the two chunk workers of a shard) get a session each ---------------- */
+/* ---- session pool: concurrent callers (and the chunk workers of a shard) get a session each -------------------- */
 static hevce_session *pool_acquire(int device, int *slot) {
     int k;
     hevce_session *s = NULL;
@@ -144,14 +144,14 @@ typedef struct {
     int *stream_len;
     /* chunk queue shared by the shard's workers */
     int nchunk, next_chunk;
-    int *chunk_first;   /* nchunk + 1 entries */
+    int *chunk_first;   /* nchunk + 1 entries; a chunk holds at least one picture, so count + 1 are allocated */
     pthread_mutex_t qlock;
 } Shard;
 
-static long long padded_pixels(int h, int w, int max_dim) {
-    long long H = ((h < max_dim ? h : max_dim) + 31) / 32 * 32, W = ((w < max_dim ? w : max_dim) + 31) / 32 * 32;
-    return H * W;
-}
+/* the reference's clamp and padding of one picture dimension (HEVCe.c:1581-1582) */
+static int padded_dim(int v, int max_dim) { return ((v < max_dim ? v : max_dim) + 31) / 32 * 32; }
+
+static long long padded_pixels(int h, int w, int max_dim) { return (long long)padded_dim(h, max_dim) * padded_dim(w, max_dim); }
 
 /* worker: encode chunks of the shard until the queue is empty */
 static void *chunk_worker(void *arg) {
@@ -186,77 +186,67 @@ static void *chunk_worker(void *arg) {
     return NULL;
 }
 
-/* encode pictures [first, first+count) on one device */
-static void *shard_main(void *arg) {
-    Shard *sh = (Shard *)arg;
-    int done = 0, cap = 16, nworkers = 2, i, same = 1;
-    pthread_t helpers[MAX_WORKERS];
-    sh->status = 0;
-    sh->nchunk = 0;
-    sh->next_chunk = 0;
-    sh->chunk_first = (int *)malloc(sizeof(int) * (size_t)(cap + 1));
-    if (!sh->chunk_first) { sh->status = HEVCE_ERR_ARG; return NULL; }
-    pthread_mutex_init(&sh->qlock, NULL);
-    /* the kernel variant is chosen for the whole shard: its chunks share the device */
-    sh->variant = hevce_internal_choose_variant(sh->device, sh->count, sh->ysz + sh->first, sh->xsz + sh->first, sh->max_dim);
+/* Cut the shard into chunks: fills chunk_first, nchunk and max_ctas, returns the number of chunk workers. */
+static int plan_chunks(Shard *sh) {
+    const int *ys = sh->ysz + sh->first, *xs = sh->xsz + sh->first;
+    int done = 0, i, same = 1;
     for (i = 1; i < sh->count && same; i++)
-        if (sh->ysz[sh->first + i] != sh->ysz[sh->first] || sh->xsz[sh->first + i] != sh->xsz[sh->first]) same = 0;
+        if (ys[i] != ys[0] || xs[i] != xs[0]) same = 0;
+    sh->nchunk = 0;
     sh->max_ctas = 0;
-    if (same && sh->count >= 8 * 7) {
+    if (same && sh->count >= 8 * G7_GANG) {
         /* Same-size pictures: rounds of four chunks (multiples of 7 pictures) on four workers, every chunk's kernel on a
            quarter of the SMs.  The four kernels run side by side, so the copies of a chunk overlap the kernels of the
            others, and the small commit kernel that follows a chunk's decision kernel finds that chunk's SMs free (behind
            whole-device kernels it would wait for the next chunk's persistent CTAs to finish). */
-        const long long px = padded_pixels(sh->ysz[sh->first], sh->xsz[sh->first], sh->max_dim) * sh->count;
-        int rounds = (int)((px + MAX_WORKERS * CHUNK_PIXELS - 1) / (MAX_WORKERS * CHUNK_PIXELS)), per, nch, sms = hevce_internal_device_sms(sh->device);
+        const long long px = padded_pixels(ys[0], xs[0], sh->max_dim) * sh->count;
+        int rounds = (int)((px + MAX_WORKERS * CHUNK_PIXELS - 1) / (MAX_WORKERS * CHUNK_PIXELS)), per, sms = hevce_internal_device_sms(sh->device);
         if (rounds < 1) rounds = 1;
-        while ((long long)rounds * MAX_WORKERS * (CHUNK_PICTURES - 7) < sh->count) rounds++;   /* many tiny pictures: the per-chunk picture bound */
-        nch = rounds * MAX_WORKERS;
-        per = (sh->count + nch - 1) / nch;
-        per = (per + 6) / 7 * 7;
-        nworkers = MAX_WORKERS;
+        while ((long long)rounds * MAX_WORKERS * (CHUNK_PICTURES - G7_GANG) < sh->count) rounds++;   /* many tiny pictures: the per-chunk picture bound */
+        per = (sh->count + rounds * MAX_WORKERS - 1) / (rounds * MAX_WORKERS);
+        per = (per + G7_GANG - 1) / G7_GANG * G7_GANG;
         /* more than one wave: cap every chunk's grid at a quarter of the SMs (smaller shards fit side by side anyway) */
         sh->max_ctas = (sms > 0 && sh->count > WAVE_PICTURES) ? (sms + MAX_WORKERS - 1) / MAX_WORKERS : 0;
-        while (nch + 1 > cap) {
-            int *p = (int *)realloc(sh->chunk_first, sizeof(int) * (size_t)(2 * cap + 1));
-            if (!p) { sh->status = HEVCE_ERR_ARG; break; }
-            sh->chunk_first = p;
-            cap *= 2;
-        }
-        while (!sh->status && done < sh->count) {
-            sh->chunk_first[sh->nchunk++] = sh->first + done;
-            done += per < sh->count - done ? per : sh->count - done;
-        }
+        for (; done < sh->count; done += per) sh->chunk_first[sh->nchunk++] = sh->first + done;
+        sh->chunk_first[sh->nchunk] = sh->first + sh->count;
+        return MAX_WORKERS;
     }
     while (done < sh->count) {
-        int a = sh->first + done, m = 0, same_c = 1;
+        int m = 0, same_c = 1;
         long long px = 0;
         while (done + m < sh->count && m < CHUNK_PICTURES &&
-               (m == 0 || px + padded_pixels(sh->ysz[a + m], sh->xsz[a + m], sh->max_dim) <= CHUNK_PIXELS)) {
-            px += padded_pixels(sh->ysz[a + m], sh->xsz[a + m], sh->max_dim);
-            if (sh->ysz[a + m] != sh->ysz[a] || sh->xsz[a + m] != sh->xsz[a]) same_c = 0;
+               (m == 0 || px + padded_pixels(ys[done + m], xs[done + m], sh->max_dim) <= CHUNK_PIXELS)) {
+            px += padded_pixels(ys[done + m], xs[done + m], sh->max_dim);
+            if (ys[done + m] != ys[done] || xs[done + m] != xs[done]) same_c = 0;
             m++;
         }
-        /* same-size pictures: whole waves of the 7-picture variant per chunk, so no chunk ends with a nearly empty wave */
+        /* same-size pictures: whole waves of g7 per chunk, so no chunk ends with a nearly empty wave */
         if (same_c && m > WAVE_PICTURES && done + m < sh->count) m -= m % WAVE_PICTURES;
-        if (sh->nchunk == cap) {
-            int *p = (int *)realloc(sh->chunk_first, sizeof(int) * (size_t)(2 * cap + 1));
-            if (!p) { sh->status = HEVCE_ERR_ARG; break; }
-            sh->chunk_first = p;
-            cap *= 2;
-        }
-        sh->chunk_first[sh->nchunk++] = a;
+        sh->chunk_first[sh->nchunk++] = sh->first + done;
         done += m;
     }
     sh->chunk_first[sh->nchunk] = sh->first + sh->count;
-    if (!sh->status) {
-        int nh = 0;
-        if (nworkers > sh->nchunk) nworkers = sh->nchunk;
-        for (i = 1; i < nworkers; i++)
-            if (pthread_create(&helpers[nh], NULL, chunk_worker, sh) == 0) nh++;
-        chunk_worker(sh);
-        for (i = 0; i < nh; i++) pthread_join(helpers[i], NULL);
-    }
+    return 2;   /* whole-device kernels: two workers, so one chunk's copies overlap the other's kernels */
+}
+
+/* encode pictures [first, first+count) on one device */
+static void *shard_main(void *arg) {
+    Shard *sh = (Shard *)arg;
+    int nworkers, nh = 0, i;
+    pthread_t helpers[MAX_WORKERS];
+    sh->status = 0;
+    sh->next_chunk = 0;
+    sh->chunk_first = (int *)malloc(sizeof(int) * (size_t)(sh->count + 1));
+    if (!sh->chunk_first) { sh->status = HEVCE_ERR_ARG; return NULL; }
+    pthread_mutex_init(&sh->qlock, NULL);
+    /* the kernel variant is chosen for the whole shard: its chunks share the device */
+    sh->variant = hevce_internal_choose_variant(sh->device, sh->count, sh->ysz + sh->first, sh->xsz + sh->first, sh->max_dim);
+    nworkers = plan_chunks(sh);
+    if (nworkers > sh->nchunk) nworkers = sh->nchunk;
+    for (i = 1; i < nworkers; i++)
+        if (pthread_create(&helpers[nh], NULL, chunk_worker, sh) == 0) nh++;
+    chunk_worker(sh);
+    for (i = 0; i < nh; i++) pthread_join(helpers[i], NULL);
     pthread_mutex_destroy(&sh->qlock);
     free(sh->chunk_first);
     return NULL;
@@ -310,8 +300,8 @@ API int HEVCImageEncoderBatch(int n, unsigned char *const *pbuffers, const unsig
         if (shards[k].status && !status) status = shards[k].status;
     if (!status)
         for (i = 0; i < n; i++) {   /* size write-back (HEVCe.c:1643-1644) */
-            ysz[i] = ((ysz[i] < max_dim ? ysz[i] : max_dim) + 31) / 32 * 32;
-            xsz[i] = ((xsz[i] < max_dim ? xsz[i] : max_dim) + 31) / 32 * 32;
+            ysz[i] = padded_dim(ysz[i], max_dim);
+            xsz[i] = padded_dim(xsz[i], max_dim);
         }
     if (lens != stream_len) free(lens);
     hevce_internal_set_device(saved_device);      /* leave the caller's current device as it was */

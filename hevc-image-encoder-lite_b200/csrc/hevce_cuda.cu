@@ -10,6 +10,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <atomic>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -124,8 +125,9 @@ struct Variant {
 #endif
 Variant g_variants[] = {HEVCE_VARIANT_LIST(HEVCE_VARIANT_ROW)};
 constexpr int NVARIANT = (int)(sizeof(g_variants) / sizeof(g_variants[0]));
-int g_forced_variant = -1;     // hevce_set_variant / HEVCE_VARIANT: -1 = choose per batch
-int g_last_variant = 0;
+// set and read by any caller thread; relaxed, as no other data is published through them
+std::atomic<int> g_forced_variant{-1};   // hevce_set_variant / HEVCE_VARIANT: -1 = choose per batch
+std::atomic<int> g_last_variant{0};
 
 Tables g_host_tables;
 std::once_flag g_variants_once;
@@ -134,7 +136,7 @@ void variants_init() {
         fill_tables(g_host_tables);
         for (int v = 0; v < NVARIANT; v++) g_variants[v].info(&g_variants[v].vi);
         if (const char* env = getenv("HEVCE_VARIANT"))
-            for (int v = 0; v < NVARIANT; v++) if (!strcmp(env, g_variants[v].name)) g_forced_variant = v;
+            for (int v = 0; v < NVARIANT; v++) if (!strcmp(env, g_variants[v].name)) g_forced_variant.store(v, std::memory_order_relaxed);
     });
 }
 
@@ -189,16 +191,35 @@ long long build_gangs(const std::vector<Job>& jobs, const std::vector<int>& orde
     return makespan;
 }
 
-template <class T>
-int grow(T** p, size_t* cap, size_t need) {   // grow-only device buffer
-    if (need <= *cap) return 0;
-    if (*p) cudaFree(*p);
-    *p = nullptr;
-    *cap = 0;
-    size_t want = need + need / 8 + 256;
-    CK(cudaMalloc((void**)p, want * sizeof(T)));
-    *cap = want;
-    return 0;
+// Grow-only buffer of T in device memory, or in pinned host memory: a larger request frees the old allocation first, then
+// allocates need + need/8 + slack elements.  The buffer frees itself; its owner selects the device before it goes.
+template <class T, bool Pinned = false>
+struct GrowBuffer {
+    T* p = nullptr;
+    size_t cap = 0;
+    GrowBuffer() = default;
+    GrowBuffer(const GrowBuffer&) = delete;
+    GrowBuffer& operator=(const GrowBuffer&) = delete;
+    ~GrowBuffer() { release(); }
+    void release() {
+        if (p) Pinned ? cudaFreeHost(p) : cudaFree(p);
+        p = nullptr;
+        cap = 0;
+    }
+    int reserve(size_t need) {
+        if (need <= cap) return 0;
+        release();
+        const size_t want = need + need / 8 + (Pinned ? 4096 : 256);
+        CK(Pinned ? cudaHostAlloc((void**)&p, want * sizeof(T), cudaHostAllocDefault) : cudaMalloc((void**)&p, want * sizeof(T)));
+        cap = want;
+        return 0;
+    }
+};
+
+// the reference's clamp and padding of a picture (HEVCe.c:1581-1582)
+void set_padded_size(Job& j, int ysz, int xsz, int max_dim) {
+    j.H = (std::min(ysz, max_dim) + CTU - 1) / CTU * CTU;
+    j.W = (std::min(xsz, max_dim) + CTU - 1) / CTU * CTU;
 }
 
 }   // namespace
@@ -214,45 +235,35 @@ struct hevce_session {
     std::vector<size_t> img_off, rcon_off, out_off;
     std::vector<int> order, results;
     size_t img_total = 0, rcon_total = 0, out_total = 0;
-    // device buffers (grow-only)
-    u8 *d_img = nullptr, *d_rcon = nullptr, *d_out = nullptr;
-    size_t c_img = 0, c_rcon = 0, c_out = 0;
-    Job* d_jobs = nullptr; size_t c_jobs = 0;
-    int* d_order = nullptr; size_t c_order = 0;
-    int* d_results = nullptr; size_t c_results = 0;
-    int* d_counter = nullptr;
-    Scratch* d_slots = nullptr; size_t c_slots = 0;
-    s16 *d_glev = nullptr, *d_lev = nullptr; u8 *d_grec = nullptr, *d_line = nullptr;
-    size_t c_glev = 0, c_lev = 0, c_grec = 0, c_line = 0;
-    CtuRec* d_recs = nullptr; size_t c_recs = 0;
-    unsigned long long* d_sse = nullptr; size_t c_sse = 0;
-    u8* d_pack = nullptr; size_t c_pack = 0;
-    unsigned long long* d_packoff = nullptr; size_t c_packoff = 0;
+    GrowBuffer<u8> d_img, d_rcon, d_out, d_grec, d_line, d_pack;
+    GrowBuffer<Job> d_jobs;
+    GrowBuffer<int> d_order, d_results, d_counter;
+    GrowBuffer<Scratch> d_slots;
+    GrowBuffer<s16> d_glev, d_lev;
+    GrowBuffer<CtuRec> d_recs;
+    GrowBuffer<unsigned long long> d_sse, d_packoff;
     float quality_ms = 0.f;
     bool encoded = false;   // hevce_session_encode has run since the last configure/upload
     std::vector<size_t> ctu_off;
     int line_pitch = 0;
-    // pinned staging
-    u8* h_stage = nullptr; size_t c_stage = 0;
+    GrowBuffer<u8, true> h_stage;   // pinned staging
 };
 
-// host-side staging copies (user buffers <-> pinned memory) spread over a few threads: at 100 Mpixel/s a single
-// thread's memcpy of a 0.8 GB step is a visible part of the end-to-end time
-static int g_copy_threads = 0;   // 0 = derive from the host's core count
-extern "C" void hevce_internal_set_copy_threads(int n) { g_copy_threads = n; }
 extern "C" int hevce_internal_get_device(void) { int d = -1; return cudaGetDevice(&d) == cudaSuccess ? d : -1; }
 extern "C" void hevce_internal_set_device(int device) { if (device >= 0) cudaSetDevice(device); }
 
+// host-side staging copies (user buffers <-> pinned memory) spread over a few threads: at 100 Mpixel/s a single
+// thread's memcpy of a 0.8 GB step is a visible part of the end-to-end time
 template <class F>
 static void parallel_pictures(int n, size_t total_bytes, F&& fn) {
-    // default: the host cores shared by up to four chunk workers per device and by every visible device (one process per GPU
+    // the host cores shared by up to four chunk workers per device and by every visible device (one process per GPU
     // or one process for all of them: either way about that many workers copy at the same time)
     static const unsigned auto_threads = [] {
         int nd = 1;
         if (cudaGetDeviceCount(&nd) != cudaSuccess || nd < 1) nd = 1;
         return std::min(4u, std::max(1u, std::thread::hardware_concurrency() / (4u * (unsigned)nd)));
     }();
-    unsigned nt = g_copy_threads > 0 ? (unsigned)g_copy_threads : auto_threads;
+    unsigned nt = auto_threads;
     if (total_bytes < ((size_t)16 << 20) || n < 2 * (int)nt) nt = 1;
     if (nt == 1) { for (int i = 0; i < n; i++) fn(i); return; }
     std::vector<std::thread> th;
@@ -261,20 +272,10 @@ static void parallel_pictures(int n, size_t total_bytes, F&& fn) {
     for (auto& x : th) x.join();
 }
 
-static int stage_reserve(hevce_session* s, size_t need) {
-    if (need <= s->c_stage) return 0;
-    if (s->h_stage) cudaFreeHost(s->h_stage);
-    s->h_stage = nullptr;
-    s->c_stage = 0;
-    CK(cudaHostAlloc((void**)&s->h_stage, need + need / 8 + 4096, cudaHostAllocDefault));
-    s->c_stage = need + need / 8 + 4096;
-    return 0;
-}
-
 // The variant (index into the variant table) that finishes these pictures soonest on one device by the
 // longest-processing-time estimate: makespan over the SMs in CTUs x the variant's measured time per CTU.
 static int choose_variant(int sms, const std::vector<Job>& jobs, const std::vector<int>& order) {
-    int best = g_forced_variant;
+    int best = g_forced_variant.load(std::memory_order_relaxed);
     if (best >= 0) return best;
     double best_t = 0;
     for (int v = 0; v < NVARIANT; v++) {
@@ -301,10 +302,7 @@ static void size_order(const std::vector<Job>& jobs, std::vector<int>& order) { 
 extern "C" int hevce_internal_choose_variant(int device, int n, const int* ysz, const int* xsz, int max_dim) {
     if (device_prepare(device) || n <= 0) return -1;
     std::vector<Job> jobs((size_t)n);
-    for (int i = 0; i < n; i++) {
-        jobs[i].H = (std::min(ysz[i], max_dim) + CTU - 1) / CTU * CTU;
-        jobs[i].W = (std::min(xsz[i], max_dim) + CTU - 1) / CTU * CTU;
-    }
+    for (int i = 0; i < n; i++) set_padded_size(jobs[i], ysz[i], xsz[i], max_dim);
     std::vector<int> order;
     size_order(jobs, order);
     return choose_variant(g_dev[device].sms, jobs, order);
@@ -330,8 +328,7 @@ extern "C" int hevce_session_configure(hevce_session* s, int n, const int* ysz, 
         if (ysz[i] <= 0 || xsz[i] <= 0 || qpd6[i] < 0 || qpd6[i] > 4) return HEVCE_ERR_ARG;
         Job& j = s->jobs[i];
         j.src_h = ysz[i]; j.src_w = xsz[i];
-        j.H = (std::min(ysz[i], max_dim) + CTU - 1) / CTU * CTU;     // HEVCe.c:1581-1582
-        j.W = (std::min(xsz[i], max_dim) + CTU - 1) / CTU * CTU;
+        set_padded_size(j, ysz[i], xsz[i], max_dim);
         j.q = qpd6[i];
         j.out_cap = 256 + 2 * j.H * j.W;
         s->img_off[i] = io; s->rcon_off[i] = ro; s->out_off[i] = oo; s->ctu_off[i] = co;
@@ -357,39 +354,39 @@ extern "C" int hevce_session_configure(hevce_session* s, int n, const int* ysz, 
     build_gangs(s->jobs, s->order, GANGV, di.sms / CLV, &gangs);
     s->ngangs = (int)gangs.size() / GANGV;
     s->grid = std::min(s->ngangs, std::max(1, (max_ctas > 0 ? std::min(max_ctas, di.sms) : di.sms) / CLV)) * CLV;
-    if ((rc = grow(&s->d_img, &s->c_img, io))) return rc;
-    if ((rc = grow(&s->d_rcon, &s->c_rcon, ro))) return rc;
-    if ((rc = grow(&s->d_out, &s->c_out, oo))) return rc;
-    if ((rc = grow(&s->d_jobs, &s->c_jobs, (size_t)n))) return rc;
-    if ((rc = grow(&s->d_order, &s->c_order, gangs.size()))) return rc;
-    if ((rc = grow(&s->d_results, &s->c_results, (size_t)2 * n))) return rc;
-    if (!s->d_counter) CK(cudaMalloc((void**)&s->d_counter, sizeof(int)));
+    if ((rc = s->d_img.reserve(io))) return rc;
+    if ((rc = s->d_rcon.reserve(ro))) return rc;
+    if ((rc = s->d_out.reserve(oo))) return rc;
+    if ((rc = s->d_jobs.reserve((size_t)n))) return rc;
+    if ((rc = s->d_order.reserve(gangs.size()))) return rc;
+    if ((rc = s->d_results.reserve((size_t)2 * n))) return rc;
+    if ((rc = s->d_counter.reserve(1))) return rc;
     const size_t g = (size_t)(s->grid / CLV) * GANGV * g_variants[best].vi.tracks, nlev = (size_t)NCAND * LEV_STRIDE + 64, nrec = (size_t)NREC * CTU * CTU;
     s->line_pitch = maxW / 4 + 32;
-    if ((rc = grow(&s->d_glev, &s->c_glev, g * nlev))) return rc;
-    if ((rc = grow(&s->d_grec, &s->c_grec, g * nrec))) return rc;
-    if ((rc = grow(&s->d_lev, &s->c_lev, co * CTU * CTU))) return rc;
-    if ((rc = grow(&s->d_recs, &s->c_recs, co))) return rc;
-    if ((rc = grow(&s->d_line, &s->c_line, g * (size_t)s->line_pitch))) return rc;
-    if ((rc = grow(&s->d_slots, &s->c_slots, g))) return rc;
+    if ((rc = s->d_glev.reserve(g * nlev))) return rc;
+    if ((rc = s->d_grec.reserve(g * nrec))) return rc;
+    if ((rc = s->d_lev.reserve(co * CTU * CTU))) return rc;
+    if ((rc = s->d_recs.reserve(co))) return rc;
+    if ((rc = s->d_line.reserve(g * (size_t)s->line_pitch))) return rc;
+    if ((rc = s->d_slots.reserve(g))) return rc;
     std::vector<Scratch> slots(g);
     for (size_t k = 0; k < g; k++) {
-        slots[k].glev = s->d_glev + k * nlev;
-        slots[k].grec = s->d_grec + k * nrec;
-        slots[k].msz_line = s->d_line + k * (size_t)s->line_pitch;
+        slots[k].glev = s->d_glev.p + k * nlev;
+        slots[k].grec = s->d_grec.p + k * nrec;
+        slots[k].msz_line = s->d_line.p + k * (size_t)s->line_pitch;
     }
     for (int i = 0; i < n; i++) {
         Job& j = s->jobs[i];
-        j.img = s->d_img + s->img_off[i];
-        j.rcon = s->d_rcon + s->rcon_off[i];
-        j.out = s->d_out + s->out_off[i];
-        j.result = s->d_results + 2 * i;
-        j.recs = s->d_recs + s->ctu_off[i];
-        j.levs = s->d_lev + s->ctu_off[i] * CTU * CTU;
+        j.img = s->d_img.p + s->img_off[i];
+        j.rcon = s->d_rcon.p + s->rcon_off[i];
+        j.out = s->d_out.p + s->out_off[i];
+        j.result = s->d_results.p + 2 * i;
+        j.recs = s->d_recs.p + s->ctu_off[i];
+        j.levs = s->d_lev.p + s->ctu_off[i] * CTU * CTU;
     }
-    CK(cudaMemcpyAsync(s->d_slots, slots.data(), g * sizeof(Scratch), cudaMemcpyHostToDevice, s->stream));
-    CK(cudaMemcpyAsync(s->d_jobs, s->jobs.data(), (size_t)n * sizeof(Job), cudaMemcpyHostToDevice, s->stream));
-    CK(cudaMemcpyAsync(s->d_order, gangs.data(), gangs.size() * sizeof(int), cudaMemcpyHostToDevice, s->stream));
+    CK(cudaMemcpyAsync(s->d_slots.p, slots.data(), g * sizeof(Scratch), cudaMemcpyHostToDevice, s->stream));
+    CK(cudaMemcpyAsync(s->d_jobs.p, s->jobs.data(), (size_t)n * sizeof(Job), cudaMemcpyHostToDevice, s->stream));
+    CK(cudaMemcpyAsync(s->d_order.p, gangs.data(), gangs.size() * sizeof(int), cudaMemcpyHostToDevice, s->stream));
     CK(cudaStreamSynchronize(s->stream));
     return 0;
 }
@@ -409,7 +406,7 @@ extern "C" hevce_session* hevce_session_create_empty(int device) {
 
 extern "C" hevce_session* hevce_session_create(int device, int n, const int* ysz, const int* xsz, const int* qpd6) {
     hevce_session* s = hevce_session_create_empty(device);
-    if (s && hevce_session_configure(s, n, ysz, xsz, qpd6, hevce_internal_max_dim(), -1, 0)) { hevce_session_destroy(s); return nullptr; }
+    if (s && hevce_session_configure(s, n, ysz, xsz, qpd6, hevce_get_max_dim(), -1, 0)) { hevce_session_destroy(s); return nullptr; }
     return s;
 }
 
@@ -417,15 +414,15 @@ extern "C" int hevce_session_upload(hevce_session* s, const unsigned char* const
     if (!s || (s->n > 0 && !imgs)) return HEVCE_ERR_ARG;
     CK(cudaSetDevice(s->device));
     if (s->n == 0) return 0;
-    int rc = stage_reserve(s, s->img_total);
+    int rc = s->h_stage.reserve(s->img_total);
     if (rc) return rc;
     for (int i = 0; i < s->n; i++)
         if (!imgs[i]) return HEVCE_ERR_ARG;
     parallel_pictures(s->n, s->img_total, [&](int i) {
         const Job& j = s->jobs[i];
-        memcpy(s->h_stage + s->img_off[i], imgs[i], (size_t)std::min(j.src_h, j.H) * j.src_w);
+        memcpy(s->h_stage.p + s->img_off[i], imgs[i], (size_t)std::min(j.src_h, j.H) * j.src_w);
     });
-    CK(cudaMemcpyAsync(s->d_img, s->h_stage, s->img_total, cudaMemcpyHostToDevice, s->stream));
+    CK(cudaMemcpyAsync(s->d_img.p, s->h_stage.p, s->img_total, cudaMemcpyHostToDevice, s->stream));
     CK(cudaStreamSynchronize(s->stream));
     s->h2d = (long long)s->img_total;
     s->encoded = false;
@@ -436,15 +433,15 @@ extern "C" int hevce_session_encode(hevce_session* s) {
     if (!s) return HEVCE_ERR_ARG;
     CK(cudaSetDevice(s->device));
     if (s->n == 0) return 0;
-    CK(cudaMemsetAsync(s->d_counter, 0, sizeof(int), s->stream));
-    CK(cudaMemsetAsync(s->d_results, 0, 2 * (size_t)s->n * sizeof(int), s->stream));
+    CK(cudaMemsetAsync(s->d_counter.p, 0, sizeof(int), s->stream));
+    CK(cudaMemsetAsync(s->d_results.p, 0, 2 * (size_t)s->n * sizeof(int), s->stream));
     CK(cudaEventRecord(s->ev0, s->stream));
-    CK((cudaError_t)g_variants[s->variant].launch(s->d_jobs, s->d_order, s->ngangs, s->d_slots, s->d_counter, g_dev[s->device].d_tables, s->grid, s->stream));
-    g_last_variant = s->variant;
+    CK((cudaError_t)g_variants[s->variant].launch(s->d_jobs.p, s->d_order.p, s->ngangs, s->d_slots.p, s->d_counter.p, g_dev[s->device].d_tables, s->grid, s->stream));
+    g_last_variant.store(s->variant, std::memory_order_relaxed);
     CK(cudaEventRecord(s->ev1, s->stream));
     {
         const dim3 grid((unsigned)((s->max_nctu + NTC - 1) / NTC), (unsigned)s->n);
-        hevce_commit_kernel<<<grid, NTC, sizeof(CommitShared), s->stream>>>(s->d_jobs, g_dev[s->device].d_tables);
+        hevce_commit_kernel<<<grid, NTC, sizeof(CommitShared), s->stream>>>(s->d_jobs.p, g_dev[s->device].d_tables);
         CK(cudaGetLastError());
     }
     CK(cudaEventRecord(s->ev2, s->stream));
@@ -461,7 +458,7 @@ extern "C" int hevce_session_download(hevce_session* s, unsigned char* const* pb
     CK(cudaSetDevice(s->device));
     if (s->n == 0) return 0;
     s->results.resize(2 * (size_t)s->n);
-    CK(cudaMemcpyAsync(s->results.data(), s->d_results, 2 * (size_t)s->n * sizeof(int), cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaMemcpyAsync(s->results.data(), s->d_results.p, 2 * (size_t)s->n * sizeof(int), cudaMemcpyDeviceToHost, s->stream));
     CK(cudaStreamSynchronize(s->stream));
     size_t bytes = 0;
     int status = 0;
@@ -473,7 +470,7 @@ extern "C" int hevce_session_download(hevce_session* s, unsigned char* const* pb
         }
         bytes += ((size_t)s->results[2 * i] + 15) & ~(size_t)15;
     }
-    int rc = stage_reserve(s, s->rcon_total + bytes);
+    int rc = s->h_stage.reserve(s->rcon_total + bytes);
     if (rc) return rc;
     // gather the streams on the device (hevce_pack_kernel), then one copy per direction: reconstructions, streams
     std::vector<unsigned long long> poff((size_t)s->n);
@@ -486,20 +483,20 @@ extern "C" int hevce_session_download(hevce_session* s, unsigned char* const* pb
         off += ((size_t)s->results[2 * i] + 15) & ~(size_t)15;
         if (stream_len) stream_len[i] = s->results[2 * i];
     }
-    if ((rc = grow(&s->d_pack, &s->c_pack, bytes + 16))) return rc;
-    if ((rc = grow(&s->d_packoff, &s->c_packoff, (size_t)s->n))) return rc;
-    CK(cudaMemcpyAsync(s->d_packoff, poff.data(), (size_t)s->n * sizeof(unsigned long long), cudaMemcpyHostToDevice, s->stream));
-    hevce_pack_kernel<<<s->n, 256, 0, s->stream>>>(s->d_jobs, s->d_packoff, s->d_results, s->d_pack);
+    if ((rc = s->d_pack.reserve(bytes + 16))) return rc;
+    if ((rc = s->d_packoff.reserve((size_t)s->n))) return rc;
+    CK(cudaMemcpyAsync(s->d_packoff.p, poff.data(), (size_t)s->n * sizeof(unsigned long long), cudaMemcpyHostToDevice, s->stream));
+    hevce_pack_kernel<<<s->n, 256, 0, s->stream>>>(s->d_jobs.p, s->d_packoff.p, s->d_results.p, s->d_pack.p);
     CK(cudaGetLastError());
     s->launches += 1;
-    CK(cudaMemcpyAsync(s->h_stage, s->d_rcon, s->rcon_total, cudaMemcpyDeviceToHost, s->stream));
-    if (bytes) CK(cudaMemcpyAsync(s->h_stage + s->rcon_total, s->d_pack, bytes, cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaMemcpyAsync(s->h_stage.p, s->d_rcon.p, s->rcon_total, cudaMemcpyDeviceToHost, s->stream));
+    if (bytes) CK(cudaMemcpyAsync(s->h_stage.p + s->rcon_total, s->d_pack.p, bytes, cudaMemcpyDeviceToHost, s->stream));
     CK(cudaStreamSynchronize(s->stream));
     off += s->rcon_total;
     parallel_pictures(s->n, off, [&](int i) {
         const Job& j = s->jobs[i];
-        memcpy(img_rcons[i], s->h_stage + s->rcon_off[i], (size_t)j.H * j.W);
-        memcpy(pbuffers[i], s->h_stage + soff[i], (size_t)s->results[2 * i]);
+        memcpy(img_rcons[i], s->h_stage.p + s->rcon_off[i], (size_t)j.H * j.W);
+        memcpy(pbuffers[i], s->h_stage.p + soff[i], (size_t)s->results[2 * i]);
     });
     s->d2h = (long long)(s->rcon_total + bytes + 2 * (size_t)s->n * sizeof(int));
     return status;
@@ -511,18 +508,18 @@ extern "C" int hevce_session_quality(hevce_session* s, double* mse, double* psnr
     if (s->n > 0 && !s->encoded) return HEVCE_ERR_STATE;   // nothing has been encoded yet
     CK(cudaSetDevice(s->device));
     if (s->n == 0) return 0;
-    int rc = grow(&s->d_sse, &s->c_sse, (size_t)s->n);
+    int rc = s->d_sse.reserve((size_t)s->n);
     if (rc) return rc;
-    CK(cudaMemsetAsync(s->d_sse, 0, (size_t)s->n * sizeof(unsigned long long), s->stream));
+    CK(cudaMemsetAsync(s->d_sse.p, 0, (size_t)s->n * sizeof(unsigned long long), s->stream));
     long long maxpix = 0;
     for (const Job& j : s->jobs) maxpix = std::max(maxpix, (long long)j.H * j.W);
     const dim3 grid((unsigned)std::max(1LL, std::min(1024LL, (maxpix / 16 + 255) / 256)), (unsigned)s->n);
     CK(cudaEventRecord(s->ev0, s->stream));
-    hevce_quality_kernel<<<grid, 256, 0, s->stream>>>(s->d_jobs, s->d_sse);
+    hevce_quality_kernel<<<grid, 256, 0, s->stream>>>(s->d_jobs.p, s->d_sse.p);
     CK(cudaGetLastError());
     CK(cudaEventRecord(s->ev1, s->stream));
     std::vector<unsigned long long> sse((size_t)s->n);
-    CK(cudaMemcpyAsync(sse.data(), s->d_sse, sse.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaMemcpyAsync(sse.data(), s->d_sse.p, sse.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
     CK(cudaStreamSynchronize(s->stream));
     CK(cudaEventElapsedTime(&s->quality_ms, s->ev0, s->ev1));
     s->launches += 1;
@@ -545,7 +542,7 @@ extern "C" int hevce_session_partition(hevce_session* s, int i, unsigned char* c
     CK(cudaSetDevice(s->device));
     const Job& j = s->jobs[i];
     std::vector<CtuRec> recs((size_t)(j.H / CTU) * (j.W / CTU));
-    CK(cudaMemcpyAsync(recs.data(), s->d_recs + s->ctu_off[i], recs.size() * sizeof(CtuRec), cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaMemcpyAsync(recs.data(), s->d_recs.p + s->ctu_off[i], recs.size() * sizeof(CtuRec), cudaMemcpyDeviceToHost, s->stream));
     CK(cudaStreamSynchronize(s->stream));
     unpack_partition(recs.data(), j.H, j.W, cu_size, mode, kind);
     return 0;
@@ -561,26 +558,17 @@ extern "C" const char* hevce_session_variant(const hevce_session* s) { return s 
 // choose per batch.  returns 0, or HEVCE_ERR_ARG for an unknown name.
 extern "C" int hevce_set_variant(const char* name) {
     variants_init();
-    if (!name || !*name || !strcmp(name, "auto")) { g_forced_variant = -1; return 0; }
+    if (!name || !*name || !strcmp(name, "auto")) { g_forced_variant.store(-1, std::memory_order_relaxed); return 0; }
     for (int v = 0; v < NVARIANT; v++)
-        if (!strcmp(name, g_variants[v].name)) { g_forced_variant = v; return 0; }
+        if (!strcmp(name, g_variants[v].name)) { g_forced_variant.store(v, std::memory_order_relaxed); return 0; }
     return HEVCE_ERR_ARG;
 }
 extern "C" long long hevce_session_h2d_bytes(const hevce_session* s) { return s ? s->h2d : 0; }
 extern "C" long long hevce_session_d2h_bytes(const hevce_session* s) { return s ? s->d2h : 0; }
 
-extern "C" void hevce_session_padded_size(const hevce_session* s, int i, int* H, int* W) {
-    *H = s->jobs[i].H;
-    *W = s->jobs[i].W;
-}
-
 extern "C" void hevce_session_destroy(hevce_session* s) {
     if (!s) return;
     cudaSetDevice(s->device);
-    cudaFree(s->d_img); cudaFree(s->d_rcon); cudaFree(s->d_out); cudaFree(s->d_jobs); cudaFree(s->d_order);
-    cudaFree(s->d_results); cudaFree(s->d_counter); cudaFree(s->d_slots); cudaFree(s->d_glev); cudaFree(s->d_grec);
-    cudaFree(s->d_lev); cudaFree(s->d_line); cudaFree(s->d_recs); cudaFree(s->d_sse); cudaFree(s->d_pack); cudaFree(s->d_packoff);
-    if (s->h_stage) cudaFreeHost(s->h_stage);
     if (s->ev0) cudaEventDestroy(s->ev0);
     if (s->ev1) cudaEventDestroy(s->ev1);
     if (s->ev2) cudaEventDestroy(s->ev2);
@@ -591,8 +579,9 @@ extern "C" void hevce_session_destroy(hevce_session* s) {
 #if defined(HEVCE_PROFILE_DUMP)
 extern "C" __attribute__((visibility("default"))) void hevce_profile_dump(void) {
     unsigned long long c[128], n[128];
-    g_variants[g_last_variant].profile(c, n);
-    printf("variant %s\n", g_variants[g_last_variant].name);
+    const Variant& last = g_variants[g_last_variant.load(std::memory_order_relaxed)];
+    last.profile(c, n);
+    printf("variant %s\n", last.name);
     static const char* names[] = {"border", "A", "B", "C", "D+pu/trial", "pu_argmin", "trial(S>8)", "decide", "adopt", "enter", "load", "commit", "misc", "teamA/round", "teamB pixel", "teamB d+cabac", "teamB argmin"};
     unsigned long long tot = 0;
     for (int i = 0; i < P_TA; i++) tot += c[i];   // team tags overlap "D+pu/trial" of the 8x8 nodes

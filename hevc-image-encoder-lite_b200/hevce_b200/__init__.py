@@ -108,9 +108,9 @@ def _out_buffers(shapes, limit):
     return outs, rcons
 
 
-def HEVCImageEncoder(img, qpd6, max_dim=None):
+def HEVCImageEncoder(img, qpd6):
     """One picture through the drop-in C entry point. Returns (stream bytes, reconstruction HxW uint8).
-    Output buffers are sized from the library's own size limit (hevce_get_max_dim), not from an argument."""
+    Output buffers are sized from the library's own size limit (hevce_get_max_dim)."""
     max_dim = get_max_dim()
     img = np.ascontiguousarray(img, dtype=np.uint8)
     if img.ndim != 2:
@@ -125,13 +125,13 @@ def HEVCImageEncoder(img, qpd6, max_dim=None):
     return out[:n].tobytes(), rcon
 
 
-def alloc_outputs(shapes, max_dim=None):
+def alloc_outputs(shapes):
     """Caller-owned output buffers (stream, reconstruction) for pictures of the given shapes; reusable across calls,
     exactly like the pbuffer / img_rcon arrays a C caller keeps."""
     return _out_buffers(shapes, get_max_dim())
 
 
-def HEVCImageEncoderBatch(imgs, qpd6, max_dim=None, outputs=None, copy_streams=True):
+def HEVCImageEncoderBatch(imgs, qpd6, outputs=None, copy_streams=True):
     """n pictures in one call (sharded over the selected GPUs). qpd6: int or sequence. Returns (streams, recons).
     outputs: buffers from alloc_outputs() to reuse; copy_streams=False returns views into them instead of bytes."""
     imgs = [np.ascontiguousarray(i, dtype=np.uint8) for i in imgs]
@@ -192,7 +192,7 @@ def measure_int_peak(device=0):
 class Session:
     """Device-resident batch on one GPU: upload once, encode (timed with CUDA events), download."""
 
-    def __init__(self, device, shapes, qpd6, max_dim=None):
+    def __init__(self, device, shapes, qpd6):
         n = len(shapes)
         self.n, self.shapes, self.max_dim = n, list(shapes), get_max_dim()
         qs = [int(qpd6)] * n if np.isscalar(qpd6) else [int(q) for q in qpd6]

@@ -160,7 +160,7 @@ def test_raised_limit_extension(H):
     strip = np.clip(np.cumsum(rng.integers(-2, 3, (33, 8243)), axis=1) + 100, 0, 255).astype(np.uint8)
     old = H.set_max_dim(16384)
     try:
-        s, r = H.HEVCImageEncoder(strip, 2, max_dim=16384)
+        s, r = H.HEVCImageEncoder(strip, 2)
     finally:
         H.set_max_dim(old)
     lib = R._load(xl)
