@@ -4,6 +4,7 @@
  *   HEVCImageEncoder       drop-in for the reference entry point (HEVCe.h:5-12, HEVCe.c:1570-1647)
  *   HEVCImageEncoderBatch  n independent pictures, sharded over the selected GPUs by cumulative CTU count,
  *                          no collective (SURVEY.md section 8e)
+ *   HEVCImageEncoderBatchDecoded  the same, plus every picture after the in-loop deblocking filter
  *
  * A shard (the pictures of one device) is cut into chunks; same-size pictures run as rounds of four chunks on four host
  * threads, each with its own session (stream + pinned staging) and its kernel on a quarter of the SMs, so the
@@ -21,6 +22,11 @@
 #include "hevce_internal.h"
 
 #define API __attribute__((visibility("default")))
+
+/* Only HEVCImageEncoderBatchDecoded reaches these two.  Weak references let this file link with a CUDA layer that does not
+   define them, such as the CPU stand-in of the chunk-planner test; in libhevce_b200.so hevce_cuda.cu defines both. */
+#pragma weak hevce_session_deblock
+#pragma weak hevce_session_download_decoded
 #define MAX_DEV 64
 #define POOL_PER_DEV 4                        /* cached sessions (grow-only buffers) per device ordinal */
 #define CHUNK_PIXELS (768LL * 1024 * 1024)    /* per-chunk bound (padded pixels) so the pinned staging stays modest */
@@ -140,6 +146,7 @@ typedef struct {
     unsigned char *const *pbuffers;
     const unsigned char *const *imgs;
     unsigned char *const *rcons;
+    unsigned char *const *decs;   /* decoded pictures, or NULL: HEVCImageEncoderBatch */
     const int *ysz, *xsz, *qpd6;
     int *stream_len;
     /* chunk queue shared by the shard's workers */
@@ -176,6 +183,8 @@ static void *chunk_worker(void *arg) {
         if (!rc) rc = hevce_session_upload(s, sh->imgs + a);
         if (!rc) rc = hevce_session_encode(s);
         if (!rc) rc = hevce_session_download(s, sh->pbuffers + a, sh->rcons + a, sh->stream_len + a);
+        if (!rc && sh->decs) rc = hevce_session_deblock(s);
+        if (!rc && sh->decs) rc = hevce_session_download_decoded(s, sh->decs + a);
         if (rc) {
             pthread_mutex_lock(&sh->qlock);
             if (!sh->status) sh->status = rc;
@@ -252,8 +261,9 @@ static void *shard_main(void *arg) {
     return NULL;
 }
 
-API int HEVCImageEncoderBatch(int n, unsigned char *const *pbuffers, const unsigned char *const *imgs,
-                              unsigned char *const *img_rcons, int *ysz, int *xsz, const int *qpd6, int *stream_len) {
+/* both batch entry points; img_decs NULL: no decoded pictures */
+static int encode_batch(int n, unsigned char *const *pbuffers, const unsigned char *const *imgs, unsigned char *const *img_rcons,
+                        unsigned char *const *img_decs, int *ysz, int *xsz, const int *qpd6, int *stream_len) {
     Shard shards[MAX_DEV];
     pthread_t threads[MAX_DEV];
     int ndev, devs[MAX_DEV], started[MAX_DEV], i, k, nshard = 0, status = 0, *lens = stream_len, saved_device;
@@ -285,7 +295,7 @@ API int HEVCImageEncoderBatch(int n, unsigned char *const *pbuffers, const unsig
         while (i < n && (k == ndev - 1 || acc + padded_pixels(ysz[i], xsz[i], max_dim) / 2 <= want)) acc += padded_pixels(ysz[i], xsz[i], max_dim), i++;
         if (i == first) continue;
         shards[nshard].device = devs[k]; shards[nshard].first = first; shards[nshard].count = i - first; shards[nshard].max_dim = max_dim;
-        shards[nshard].pbuffers = pbuffers; shards[nshard].imgs = imgs; shards[nshard].rcons = img_rcons;
+        shards[nshard].pbuffers = pbuffers; shards[nshard].imgs = imgs; shards[nshard].rcons = img_rcons; shards[nshard].decs = img_decs;
         shards[nshard].ysz = ysz; shards[nshard].xsz = xsz; shards[nshard].qpd6 = qpd6; shards[nshard].stream_len = lens;
         nshard++;
     }
@@ -306,6 +316,21 @@ API int HEVCImageEncoderBatch(int n, unsigned char *const *pbuffers, const unsig
     if (lens != stream_len) free(lens);
     hevce_internal_set_device(saved_device);      /* leave the caller's current device as it was */
     return status;
+}
+
+API int HEVCImageEncoderBatch(int n, unsigned char *const *pbuffers, const unsigned char *const *imgs,
+                              unsigned char *const *img_rcons, int *ysz, int *xsz, const int *qpd6, int *stream_len) {
+    return encode_batch(n, pbuffers, imgs, img_rcons, NULL, ysz, xsz, qpd6, stream_len);
+}
+
+API int HEVCImageEncoderBatchDecoded(int n, unsigned char *const *pbuffers, const unsigned char *const *imgs, unsigned char *const *img_rcons,
+                                     unsigned char *const *img_decs, int *ysz, int *xsz, const int *qpd6, int *stream_len) {
+    int i;
+    if (!hevce_session_deblock || !hevce_session_download_decoded) return HEVCE_ERR_STATE;   /* linked without them */
+    if (n > 0 && !img_decs) return HEVCE_ERR_ARG;
+    for (i = 0; i < n; i++)
+        if (!img_decs[i]) return HEVCE_ERR_ARG;
+    return encode_batch(n, pbuffers, imgs, img_rcons, img_decs, ysz, xsz, qpd6, stream_len);
 }
 
 API int HEVCImageEncoder(unsigned char *pbuffer, const unsigned char *img, unsigned char *img_rcon, int *ysz, int *xsz, const int qpd6) {

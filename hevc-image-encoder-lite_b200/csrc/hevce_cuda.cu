@@ -22,6 +22,7 @@
 
 #include "../../include/hevce.h"
 #include "hevce_core.h"
+#include "hevce_deblock.h"
 #include "hevce_internal.h"
 #include "hevce_variants.h"
 
@@ -62,13 +63,13 @@ __global__ void __launch_bounds__(256) hevce_pack_kernel(const Job* __restrict__
 
 // Quality pass (HEVCeMain.c:116-133): sum of squared differences between source and reconstruction over the area both
 // cover.  blockIdx.y = picture, a CTA strides over 16-pixel segments of the reconstruction rows.  HBM-bound: 2 B/pixel.
-__global__ void __launch_bounds__(256) hevce_quality_kernel(const Job* __restrict__ jobs, unsigned long long* __restrict__ sse) {
-    const Job job = jobs[blockIdx.y];
+// `plane` is the picture's H x W plane to compare: its reconstruction, or the decoded picture at the same offset.
+__device__ __forceinline__ void quality_sse(const Job& job, const u8* __restrict__ plane, unsigned long long* __restrict__ sse) {
     const int hm = min(job.src_h, job.H), wm = min(job.src_w, job.W), segs = (wm + 15) / 16;
     unsigned long long acc = 0;
     for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < (long long)hm * segs; t += (long long)gridDim.x * blockDim.x) {
         const int y = (int)(t / segs), x0 = (int)(t % segs) * 16;
-        const uint4 rv = *(const uint4*)(job.rcon + (size_t)y * job.W + x0);   // rows of the reconstruction are 32-byte aligned
+        const uint4 rv = *(const uint4*)(plane + (size_t)y * job.W + x0);   // rows of the plane are 32-byte aligned
         const u32 rw[4] = {rv.x, rv.y, rv.z, rv.w};
         const u8* ip = job.img + (size_t)y * job.src_w + x0;
         unsigned part = 0;
@@ -83,6 +84,37 @@ __global__ void __launch_bounds__(256) hevce_quality_kernel(const Job* __restric
     }
     for (int o = 16; o > 0; o >>= 1) acc += __shfl_down_sync(0xffffffffu, acc, o);
     if ((threadIdx.x & 31) == 0 && acc) atomicAdd(sse + blockIdx.y, acc);
+}
+
+__global__ void __launch_bounds__(256) hevce_quality_kernel(const Job* __restrict__ jobs, unsigned long long* __restrict__ sse) {
+    const Job job = jobs[blockIdx.y];
+    quality_sse(job, job.rcon, sse);
+}
+
+// the same over the decoded pictures: dec_base holds each picture at its reconstruction's offset from rcon_base
+__global__ void __launch_bounds__(256) hevce_decoded_quality_kernel(const Job* __restrict__ jobs, const u8* rcon_base, const u8* dec_base,
+                                                                    unsigned long long* __restrict__ sse) {
+    const Job job = jobs[blockIdx.y];
+    quality_sse(job, dec_base + (job.rcon - rcon_base), sse);
+}
+
+// In-loop deblocking filter (hevce_deblock.h): one CTA per (CTU, picture), blockIdx.y = picture.  Reads the
+// reconstructions, writes the decoded pictures to dec_base at the reconstructions' offsets from rcon_base.
+__global__ void __launch_bounds__(DBK_THREADS) hevce_deblock_kernel(const Job* __restrict__ jobs, const u8* rcon_base, u8* dec_base) {
+    __shared__ DbkTile t;
+    const Job job = jobs[blockIdx.y];
+    const int ctu = blockIdx.x;
+    if (ctu >= dbk_nctu(job)) return;
+    for (int i = threadIdx.x; i < DBK_LOAD_ITEMS; i += DBK_THREADS) dbk_load(t, job, ctu, i);
+    __syncthreads();
+    if (dbk_active(job)) {
+        for (int i = threadIdx.x; i < DBK_VERT_ITEMS; i += DBK_THREADS) dbk_vertical(t, job, ctu, i);
+        __syncthreads();
+        for (int i = threadIdx.x; i < DBK_HORZ_ITEMS; i += DBK_THREADS) dbk_horizontal(t, job, ctu, i);
+        __syncthreads();
+    }
+    u8* dec = dec_base + (job.rcon - rcon_base);
+    for (int i = threadIdx.x; i < DBK_STORE_ITEMS; i += DBK_THREADS) dbk_store(t, job, ctu, dec, i);
 }
 
 // integer-issue micro-benchmark: 8 independent IMAD chains + 8 independent LOP3/IADD3 chains per thread
@@ -242,8 +274,10 @@ struct hevce_session {
     GrowBuffer<s16> d_glev, d_lev;
     GrowBuffer<CtuRec> d_recs;
     GrowBuffer<unsigned long long> d_sse, d_packoff;
-    float quality_ms = 0.f;
+    float quality_ms = 0.f, deblock_ms = 0.f;
     bool encoded = false;   // hevce_session_encode has run since the last configure/upload
+    bool deblocked = false; // hevce_session_deblock has run since the last configure/upload/encode
+    GrowBuffer<u8> d_dec;   // decoded pictures at the offsets of d_rcon; reserved by the first hevce_session_deblock
     std::vector<size_t> ctu_off;
     int line_pitch = 0;
     GrowBuffer<u8, true> h_stage;   // pinned staging
@@ -316,7 +350,7 @@ extern "C" int hevce_session_configure(hevce_session* s, int n, const int* ysz, 
     if (!s || n < 0 || n > 65535 || (n > 0 && (!ysz || !xsz || !qpd6))) return HEVCE_ERR_ARG;   // grid.y of the commit kernel = picture index
     int rc = device_prepare(s->device);
     if (rc) return rc;
-    s->encoded = false;
+    s->encoded = s->deblocked = false;
     s->n = n;
     s->jobs.assign(n, Job());
     s->img_off.assign(n, 0); s->rcon_off.assign(n, 0); s->out_off.assign(n, 0); s->ctu_off.assign(n, 0);
@@ -425,12 +459,13 @@ extern "C" int hevce_session_upload(hevce_session* s, const unsigned char* const
     CK(cudaMemcpyAsync(s->d_img.p, s->h_stage.p, s->img_total, cudaMemcpyHostToDevice, s->stream));
     CK(cudaStreamSynchronize(s->stream));
     s->h2d = (long long)s->img_total;
-    s->encoded = false;
+    s->encoded = s->deblocked = false;
     return 0;
 }
 
 extern "C" int hevce_session_encode(hevce_session* s) {
     if (!s) return HEVCE_ERR_ARG;
+    s->deblocked = false;
     CK(cudaSetDevice(s->device));
     if (s->n == 0) return 0;
     CK(cudaMemsetAsync(s->d_counter.p, 0, sizeof(int), s->stream));
@@ -502,10 +537,9 @@ extern "C" int hevce_session_download(hevce_session* s, unsigned char* const* pb
     return status;
 }
 
-// f3: per-picture MSE / PSNR of the last encode, reduced on the device (calcImagePSNR, HEVCeMain.c:116-133)
-extern "C" int hevce_session_quality(hevce_session* s, double* mse, double* psnr) {
-    if (!s || (s->n > 0 && !mse && !psnr)) return HEVCE_ERR_ARG;
-    if (s->n > 0 && !s->encoded) return HEVCE_ERR_STATE;   // nothing has been encoded yet
+// f3: per-picture MSE / PSNR against the source, reduced on the device (calcImagePSNR, HEVCeMain.c:116-133), of the
+// reconstructions or (decoded) of the decoded pictures
+static int session_quality(hevce_session* s, bool decoded, double* mse, double* psnr) {
     CK(cudaSetDevice(s->device));
     if (s->n == 0) return 0;
     int rc = s->d_sse.reserve((size_t)s->n);
@@ -515,7 +549,8 @@ extern "C" int hevce_session_quality(hevce_session* s, double* mse, double* psnr
     for (const Job& j : s->jobs) maxpix = std::max(maxpix, (long long)j.H * j.W);
     const dim3 grid((unsigned)std::max(1LL, std::min(1024LL, (maxpix / 16 + 255) / 256)), (unsigned)s->n);
     CK(cudaEventRecord(s->ev0, s->stream));
-    hevce_quality_kernel<<<grid, 256, 0, s->stream>>>(s->d_jobs.p, s->d_sse.p);
+    if (decoded) hevce_decoded_quality_kernel<<<grid, 256, 0, s->stream>>>(s->d_jobs.p, s->d_rcon.p, s->d_dec.p, s->d_sse.p);
+    else hevce_quality_kernel<<<grid, 256, 0, s->stream>>>(s->d_jobs.p, s->d_sse.p);
     CK(cudaGetLastError());
     CK(cudaEventRecord(s->ev1, s->stream));
     std::vector<unsigned long long> sse((size_t)s->n);
@@ -532,7 +567,58 @@ extern "C" int hevce_session_quality(hevce_session* s, double* mse, double* psnr
     }
     return 0;
 }
+
+extern "C" int hevce_session_quality(hevce_session* s, double* mse, double* psnr) {
+    if (!s || (s->n > 0 && !mse && !psnr)) return HEVCE_ERR_ARG;
+    if (s->n > 0 && !s->encoded) return HEVCE_ERR_STATE;   // nothing has been encoded yet
+    return session_quality(s, false, mse, psnr);
+}
 extern "C" float hevce_session_quality_ms(const hevce_session* s) { return s ? s->quality_ms : 0.f; }
+
+// f5: the decoded pictures of the last encode -- the reconstructions after the in-loop deblocking filter
+extern "C" int hevce_session_deblock(hevce_session* s) {
+    if (!s) return HEVCE_ERR_ARG;
+    if (s->n > 0 && !s->encoded) return HEVCE_ERR_STATE;   // nothing has been encoded yet
+    CK(cudaSetDevice(s->device));
+    if (s->n > 0) {
+        int rc = s->d_dec.reserve(s->rcon_total);
+        if (rc) return rc;
+        CK(cudaEventRecord(s->ev0, s->stream));
+        hevce_deblock_kernel<<<dim3((unsigned)s->max_nctu, (unsigned)s->n), DBK_THREADS, 0, s->stream>>>(s->d_jobs.p, s->d_rcon.p, s->d_dec.p);
+        CK(cudaGetLastError());
+        CK(cudaEventRecord(s->ev1, s->stream));
+        CK(cudaStreamSynchronize(s->stream));
+        CK(cudaEventElapsedTime(&s->deblock_ms, s->ev0, s->ev1));
+        s->launches += 1;
+    }
+    s->deblocked = true;
+    return 0;
+}
+extern "C" float hevce_session_deblock_ms(const hevce_session* s) { return s ? s->deblock_ms : 0.f; }
+
+extern "C" int hevce_session_download_decoded(hevce_session* s, unsigned char* const* img_decs) {
+    if (!s || (s->n > 0 && !img_decs)) return HEVCE_ERR_ARG;
+    if (s->n > 0 && !s->deblocked) return HEVCE_ERR_STATE;
+    CK(cudaSetDevice(s->device));
+    if (s->n == 0) return 0;
+    for (int i = 0; i < s->n; i++)
+        if (!img_decs[i]) return HEVCE_ERR_ARG;
+    int rc = s->h_stage.reserve(s->rcon_total);
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(s->h_stage.p, s->d_dec.p, s->rcon_total, cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaStreamSynchronize(s->stream));
+    parallel_pictures(s->n, s->rcon_total, [&](int i) {
+        const Job& j = s->jobs[i];
+        memcpy(img_decs[i], s->h_stage.p + s->rcon_off[i], (size_t)j.H * j.W);
+    });
+    return 0;
+}
+
+extern "C" int hevce_session_decoded_quality(hevce_session* s, double* mse, double* psnr) {
+    if (!s || (s->n > 0 && !mse && !psnr)) return HEVCE_ERR_ARG;
+    if (s->n > 0 && !s->deblocked) return HEVCE_ERR_STATE;
+    return session_quality(s, true, mse, psnr);
+}
 
 // Decisions of picture i after hevce_session_encode: CU size and luma intra mode per 4x4 unit ((H/4)*(W/4) bytes each),
 // CU kind per 8x8 unit ((H/8)*(W/8) bytes: 0 one TU, 1 four TUs, 2 NxN).  Any pointer may be NULL.

@@ -26,6 +26,8 @@ EXPORTS = [
     "hevce_session_h2d_bytes", "hevce_session_d2h_bytes", "hevce_session_destroy",
     "hevce_session_quality", "hevce_session_quality_ms", "hevce_session_partition",
     "hevce_set_variant", "hevce_session_variant", "hevce_get_max_dim", "hevce_release",
+    "HEVCImageEncoderBatchDecoded", "hevce_session_deblock", "hevce_session_deblock_ms", "hevce_session_download_decoded",
+    "hevce_session_decoded_quality",
 ]
 
 
@@ -50,6 +52,8 @@ def lib():
         L.HEVCImageEncoder.argtypes = [_u8p, _u8p, _u8p, _ip, _ip, ctypes.c_int]
         L.HEVCImageEncoderBatch.restype = ctypes.c_int
         L.HEVCImageEncoderBatch.argtypes = [ctypes.c_int, ctypes.POINTER(_u8p), ctypes.POINTER(_u8p), ctypes.POINTER(_u8p), _ip, _ip, _ip, _ip]
+        L.HEVCImageEncoderBatchDecoded.restype = ctypes.c_int
+        L.HEVCImageEncoderBatchDecoded.argtypes = [ctypes.c_int] + [ctypes.POINTER(_u8p)] * 4 + [_ip, _ip, _ip, _ip]
         L.hevce_set_devices.restype = ctypes.c_int
         L.hevce_set_devices.argtypes = [ctypes.c_int, _ip]
         L.hevce_set_max_dim.restype = ctypes.c_int
@@ -74,11 +78,16 @@ def lib():
         L.hevce_session_encode.argtypes = [ctypes.c_void_p]
         L.hevce_session_download.restype = ctypes.c_int
         L.hevce_session_download.argtypes = [ctypes.c_void_p, ctypes.POINTER(_u8p), ctypes.POINTER(_u8p), _ip]
-        L.hevce_session_quality.restype = ctypes.c_int
-        L.hevce_session_quality.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]
+        for f in ("hevce_session_quality", "hevce_session_decoded_quality"):
+            getattr(L, f).restype = ctypes.c_int
+            getattr(L, f).argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]
+        L.hevce_session_deblock.restype = ctypes.c_int
+        L.hevce_session_deblock.argtypes = [ctypes.c_void_p]
+        L.hevce_session_download_decoded.restype = ctypes.c_int
+        L.hevce_session_download_decoded.argtypes = [ctypes.c_void_p, ctypes.POINTER(_u8p)]
         L.hevce_session_partition.restype = ctypes.c_int
         L.hevce_session_partition.argtypes = [ctypes.c_void_p, ctypes.c_int, _u8p, _u8p, _u8p]
-        for f in ("hevce_session_kernel_ms", "hevce_session_commit_ms", "hevce_session_quality_ms"):
+        for f in ("hevce_session_kernel_ms", "hevce_session_commit_ms", "hevce_session_quality_ms", "hevce_session_deblock_ms"):
             getattr(L, f).restype = ctypes.c_float
             getattr(L, f).argtypes = [ctypes.c_void_p]
         for f in ("hevce_session_launches", "hevce_session_grid"):
@@ -153,6 +162,33 @@ def HEVCImageEncoderBatch(imgs, qpd6, outputs=None, copy_streams=True):
     if not copy_streams:
         return [outs[i][: lens[i]] for i in range(n)], rcons
     return [outs[i][: lens[i]].tobytes() for i in range(n)], rcons
+
+
+def HEVCImageEncoderBatchDecoded(imgs, qpd6, outputs=None):
+    """HEVCImageEncoderBatch that also returns the decoded pictures: the reconstructions after the in-loop deblocking
+    filter, which is what a conforming decoder shows for the streams.  Returns (streams, recons, decoded).
+    outputs: (streams, recons, decoded) buffers to reuse, e.g. alloc_outputs() plus one more list like recons."""
+    imgs = [np.ascontiguousarray(i, dtype=np.uint8) for i in imgs]
+    n = len(imgs)
+    qs = [int(qpd6)] * n if np.isscalar(qpd6) else [int(q) for q in qpd6]
+    limit = get_max_dim()
+    if outputs is not None:
+        outs, rcons, decs = outputs
+    else:
+        outs, rcons = _out_buffers([i.shape for i in imgs], limit)
+        decs = [np.zeros_like(r) for r in rcons]
+    for i, o, r, d in zip(imgs, outs, rcons, decs):   # the library clamps with ITS limit: never hand it a smaller buffer
+        need = padded(i.shape[0], limit) * padded(i.shape[1], limit)
+        if r.size < need or d.size < need or o.size < 256 + 2 * need:
+            raise HevceError(ERR_ARG, "HEVCImageEncoderBatchDecoded: output buffers smaller than the library's size limit requires")
+    ys = (ctypes.c_int * n)(*[i.shape[0] for i in imgs])
+    xs = (ctypes.c_int * n)(*[i.shape[1] for i in imgs])
+    qa = (ctypes.c_int * n)(*qs)
+    lens = (ctypes.c_int * n)()
+    rc = lib().HEVCImageEncoderBatchDecoded(n, _ptr_array(outs), _ptr_array(imgs), _ptr_array(rcons), _ptr_array(decs), ys, xs, qa, lens)
+    if rc < 0:
+        raise HevceError(rc, "HEVCImageEncoderBatchDecoded")
+    return [outs[i][: lens[i]].tobytes() for i in range(n)], rcons, decs
 
 
 def set_devices(ordinals):
@@ -240,6 +276,34 @@ class Session:
     @property
     def quality_ms(self):
         return lib().hevce_session_quality_ms(self._h)
+
+    def deblock(self):
+        """Run the in-loop deblocking filter over the last encode's reconstructions on the device; returns its kernel ms."""
+        rc = lib().hevce_session_deblock(self._h)
+        if rc < 0:
+            raise HevceError(rc, "hevce_session_deblock")
+        return lib().hevce_session_deblock_ms(self._h)
+
+    @property
+    def deblock_ms(self):
+        return lib().hevce_session_deblock_ms(self._h)
+
+    def download_decoded(self):
+        """The decoded pictures (padded, like the reconstructions) after deblock()."""
+        decs = [np.zeros((padded(h, self.max_dim), padded(w, self.max_dim)), np.uint8) for h, w in self.shapes]
+        rc = lib().hevce_session_download_decoded(self._h, _ptr_array(decs))
+        if rc < 0:
+            raise HevceError(rc, "hevce_session_download_decoded")
+        return decs
+
+    def decoded_quality(self):
+        """(mse, psnr) of every decoded picture against its source, as quality() does for the reconstructions."""
+        mse, psnr = np.zeros(self.n, np.float64), np.zeros(self.n, np.float64)
+        dp = ctypes.POINTER(ctypes.c_double)
+        rc = lib().hevce_session_decoded_quality(self._h, mse.ctypes.data_as(dp), psnr.ctypes.data_as(dp))
+        if rc < 0:
+            raise HevceError(rc, "hevce_session_decoded_quality")
+        return mse, psnr
 
     def partition(self, i):
         """Decisions of picture i: (cu_size, mode) per 4x4 unit and kind per 8x8 unit (0 one TU, 1 four TUs, 2 NxN)."""

@@ -53,6 +53,16 @@ HEVCE_API int HEVCImageEncoder(unsigned char *pbuffer, const unsigned char *img,
 HEVCE_API int HEVCImageEncoderBatch(int n, unsigned char *const *pbuffers, const unsigned char *const *imgs,
                           unsigned char *const *img_rcons, int *ysz, int *xsz, const int *qpd6, int *stream_len);
 
+/*
+ * New: HEVCImageEncoderBatch that also returns the decoded pictures: img_decs[i] receives picture i after the in-loop
+ * deblocking filter (see hevce_session_deblock), padded size, stride = padded width.  Everything else, including the
+ * split of the batch over devices and chunks, is that of HEVCImageEncoderBatch.  A NULL img_decs or img_decs[i] is
+ * HEVCE_ERR_ARG.  returns 0, or a negative HEVCE_ERR_*.
+ */
+HEVCE_API int HEVCImageEncoderBatchDecoded(int n, unsigned char *const *pbuffers, const unsigned char *const *imgs,
+                          unsigned char *const *img_rcons, unsigned char *const *img_decs, int *ysz, int *xsz,
+                          const int *qpd6, int *stream_len);
+
 /* ---- extensions used by the benchmark harness and the multi-process launcher ------------------------------ */
 
 /* Restrict the library to `count` CUDA device ordinals (default: every visible device; the environment
@@ -96,11 +106,23 @@ HEVCE_API const char *hevce_session_variant(const hevce_session *s); /* kernel v
  * reference CLI at HEVCeMain.c:201-212).  mse / psnr: n doubles each, either may be NULL.  HEVCE_ERR_STATE before the
  * first hevce_session_encode of the uploaded pictures (the same holds for hevce_session_partition). */
 HEVCE_API int  hevce_session_quality(hevce_session *s, double *mse, double *psnr);
-HEVCE_API float hevce_session_quality_ms(const hevce_session *s);  /* CUDA-event duration of the last hevce_quality_kernel launch */
+HEVCE_API float hevce_session_quality_ms(const hevce_session *s);  /* CUDA-event duration of the last quality kernel launch (this call's or hevce_session_decoded_quality's) */
 /* Decisions of picture i of the last encode as raster maps: CU size (8/16/32) and luma intra mode (0..34) per 4x4 unit,
  * (H/4)*(W/4) bytes each; CU kind per 8x8 unit, (H/8)*(W/8) bytes: 0 = one TU, 1 = four TUs, 2 = NxN (what the
  * reference keeps in map_cu_sz_0 / map_pmode_0, HEVCe.c:1591-1592, plus the transform split).  Any pointer may be NULL. */
 HEVCE_API int  hevce_session_partition(hevce_session *s, int i, unsigned char *cu_size, unsigned char *mode, unsigned char *kind);
+/* The decoded picture: the reconstruction after the in-loop deblocking filter (H.265 section 8.7.2), which the stream
+ * header leaves enabled, so it is what a conforming decoder outputs for the stream.  At qpd6 0-1 the filter changes
+ * nothing and the decoded picture equals the reconstruction.
+ * hevce_session_deblock filters the reconstructions of the last encode on the device (synchronous); HEVCE_ERR_STATE
+ * before the first hevce_session_encode of the uploaded pictures.  The other three return HEVCE_ERR_STATE unless
+ * hevce_session_deblock has run since the last configure, upload or encode.  img_decs: n buffers of the padded size,
+ * stride = padded width, like img_rcons.  hevce_session_decoded_quality: hevce_session_quality's MSE / PSNR, taken
+ * between the source and the decoded picture. */
+HEVCE_API int   hevce_session_deblock(hevce_session *s);
+HEVCE_API float hevce_session_deblock_ms(const hevce_session *s);   /* CUDA-event duration of that hevce_deblock_kernel launch */
+HEVCE_API int   hevce_session_download_decoded(hevce_session *s, unsigned char *const *img_decs);   /* HBM -> host */
+HEVCE_API int   hevce_session_decoded_quality(hevce_session *s, double *mse, double *psnr);
 HEVCE_API long long hevce_session_h2d_bytes(const hevce_session *s);
 HEVCE_API long long hevce_session_d2h_bytes(const hevce_session *s);
 HEVCE_API void hevce_session_destroy(hevce_session *s);
