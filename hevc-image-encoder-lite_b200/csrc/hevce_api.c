@@ -5,6 +5,7 @@
  *   HEVCImageEncoderBatch  n independent pictures, sharded over the selected GPUs by cumulative CTU count,
  *                          no collective (SURVEY.md section 8e)
  *   HEVCImageEncoderBatchDecoded  the same, plus every picture after the in-loop deblocking filter
+ *   HEVCImageDecoderBatch  streams of this library back to decoded pictures, sharded the same way
  *
  * A shard (the pictures of one device) is cut into chunks; same-size pictures run as rounds of four chunks on four host
  * threads, each with its own session (stream + pinned staging) and its kernel on a quarter of the SMs, so the
@@ -27,6 +28,13 @@
    define them, such as the CPU stand-in of the chunk-planner test; in libhevce_b200.so hevce_cuda.cu defines both. */
 #pragma weak hevce_session_deblock
 #pragma weak hevce_session_download_decoded
+/* The same for the decoder (HEVCImageDecoderBatch returns HEVCE_ERR_STATE without them). */
+#pragma weak hevce_stream_info
+#pragma weak hevce_decoder_create
+#pragma weak hevce_decoder_upload
+#pragma weak hevce_decoder_run
+#pragma weak hevce_decoder_download
+#pragma weak hevce_decoder_destroy
 #define MAX_DEV 64
 #define POOL_PER_DEV 4                        /* cached sessions (grow-only buffers) per device ordinal */
 #define CHUNK_PIXELS (768LL * 1024 * 1024)    /* per-chunk bound (padded pixels) so the pinned staging stays modest */
@@ -40,6 +48,8 @@ static int g_ndev = -1, g_devs[MAX_DEV];
 static int g_max_dim = 8192;
 static hevce_session *g_pool[MAX_DEV][POOL_PER_DEV];
 static int g_pool_busy[MAX_DEV][POOL_PER_DEV];
+static hevce_decoder *g_dec[MAX_DEV];   /* one cached decoder per device ordinal */
+static int g_dec_busy[MAX_DEV];
 
 API const char *hevce_version(void) { return "hevce-b200 0.2 (sm_100a)"; }
 
@@ -139,6 +149,13 @@ API void hevce_release(void) {
             pthread_mutex_unlock(&g_lock);
             if (s) hevce_session_destroy(s);
         }
+    for (d = 0; d < MAX_DEV; d++) {
+        hevce_decoder *dec = NULL;
+        pthread_mutex_lock(&g_lock);
+        if (!g_dec_busy[d]) { dec = g_dec[d]; g_dec[d] = NULL; }
+        pthread_mutex_unlock(&g_lock);
+        if (dec) hevce_decoder_destroy(dec);
+    }
 }
 
 typedef struct {
@@ -261,14 +278,32 @@ static void *shard_main(void *arg) {
     return NULL;
 }
 
+/* Contiguous shards with (nearly) equal padded-pixel = CTU counts over ndev devices: shard k holds pictures
+   [first[k], first[k] + count[k]) on device dev[k].  Returns the number of shards (devices without pictures get none). */
+static int cut_shards(int n, const int *ysz, const int *xsz, int max_dim, int ndev, const int *devs, int *dev, int *first, int *count) {
+    long long total = 0, acc = 0;
+    int i, k, nshard = 0;
+    for (i = 0; i < n; i++) total += padded_pixels(ysz[i], xsz[i], max_dim);
+    if (ndev > n) ndev = n;
+    for (k = 0, i = 0; k < ndev; k++) {
+        int f = i;
+        long long want = total * (k + 1) / ndev;
+        while (i < n && (k == ndev - 1 || acc + padded_pixels(ysz[i], xsz[i], max_dim) / 2 <= want)) acc += padded_pixels(ysz[i], xsz[i], max_dim), i++;
+        if (i == f) continue;
+        dev[nshard] = devs[k]; first[nshard] = f; count[nshard] = i - f;
+        nshard++;
+    }
+    return nshard;
+}
+
 /* both batch entry points; img_decs NULL: no decoded pictures */
 static int encode_batch(int n, unsigned char *const *pbuffers, const unsigned char *const *imgs, unsigned char *const *img_rcons,
                         unsigned char *const *img_decs, int *ysz, int *xsz, const int *qpd6, int *stream_len) {
     Shard shards[MAX_DEV];
     pthread_t threads[MAX_DEV];
     int ndev, devs[MAX_DEV], started[MAX_DEV], i, k, nshard = 0, status = 0, *lens = stream_len, saved_device;
+    int cut_dev[MAX_DEV], cut_first[MAX_DEV], cut_count[MAX_DEV];
     const int max_dim = hevce_get_max_dim();   /* one value for the whole call: sharding, clamp and size write-back */
-    long long total = 0, acc = 0;
     if (n < 0) return HEVCE_ERR_ARG;
     if (n == 0) return 0;
     if (!pbuffers || !imgs || !img_rcons || !ysz || !xsz || !qpd6) return HEVCE_ERR_ARG;
@@ -286,18 +321,11 @@ static int encode_batch(int n, unsigned char *const *pbuffers, const unsigned ch
     if (!lens) lens = (int *)malloc(sizeof(int) * (size_t)n);
     if (!lens) return HEVCE_ERR_ARG;
     saved_device = hevce_internal_get_device();   /* shard 0 runs on this thread and selects its device */
-    for (i = 0; i < n; i++) total += padded_pixels(ysz[i], xsz[i], max_dim);
-    /* contiguous shards with (nearly) equal padded-pixel = CTU counts */
-    if (ndev > n) ndev = n;
-    for (k = 0, i = 0; k < ndev; k++) {
-        int first = i;
-        long long want = total * (k + 1) / ndev;
-        while (i < n && (k == ndev - 1 || acc + padded_pixels(ysz[i], xsz[i], max_dim) / 2 <= want)) acc += padded_pixels(ysz[i], xsz[i], max_dim), i++;
-        if (i == first) continue;
-        shards[nshard].device = devs[k]; shards[nshard].first = first; shards[nshard].count = i - first; shards[nshard].max_dim = max_dim;
-        shards[nshard].pbuffers = pbuffers; shards[nshard].imgs = imgs; shards[nshard].rcons = img_rcons; shards[nshard].decs = img_decs;
-        shards[nshard].ysz = ysz; shards[nshard].xsz = xsz; shards[nshard].qpd6 = qpd6; shards[nshard].stream_len = lens;
-        nshard++;
+    nshard = cut_shards(n, ysz, xsz, max_dim, ndev, devs, cut_dev, cut_first, cut_count);
+    for (k = 0; k < nshard; k++) {
+        shards[k].device = cut_dev[k]; shards[k].first = cut_first[k]; shards[k].count = cut_count[k]; shards[k].max_dim = max_dim;
+        shards[k].pbuffers = pbuffers; shards[k].imgs = imgs; shards[k].rcons = img_rcons; shards[k].decs = img_decs;
+        shards[k].ysz = ysz; shards[k].xsz = xsz; shards[k].qpd6 = qpd6; shards[k].stream_len = lens;
     }
     for (k = 1; k < nshard; k++) {
         started[k] = pthread_create(&threads[k], NULL, shard_main, &shards[k]) == 0;
@@ -342,4 +370,104 @@ API int HEVCImageEncoder(unsigned char *pbuffer, const unsigned char *img, unsig
     pb[0] = pbuffer; im[0] = img; rc_[0] = img_rcon;
     rc = HEVCImageEncoderBatch(1, pb, im, rc_, ysz, xsz, &qpd6, &len);
     return rc ? rc : len;
+}
+
+/* ---- f6: the decoder ----------------------------------------------------------------------------------------- */
+typedef struct {
+    int device, first, count, status;
+    const unsigned char *const *streams;
+    const int *stream_len, *ysz, *xsz;
+    unsigned char *const *decs;
+    int *pic_status;
+} DecShard;
+
+/* decode pictures [first, first+count) on one device, in chunks of at most CHUNK_PIXELS / CHUNK_PICTURES; a chunk whose
+   pictures did not all parse does not stop the others */
+static void *dec_shard_main(void *arg) {
+    DecShard *sh = (DecShard *)arg;
+    hevce_decoder *d = NULL;
+    int cached = 0, done = 0;
+    sh->status = 0;
+    pthread_mutex_lock(&g_lock);
+    if (!g_dec_busy[sh->device]) { g_dec_busy[sh->device] = 1; cached = 1; d = g_dec[sh->device]; }
+    pthread_mutex_unlock(&g_lock);
+    if (!d) d = hevce_decoder_create(sh->device);   /* first use, or another call is using the cached one */
+    if (d && cached) {
+        pthread_mutex_lock(&g_lock);
+        g_dec[sh->device] = d;
+        pthread_mutex_unlock(&g_lock);
+    }
+    if (!d) sh->status = HEVCE_ERR_CUDA;
+    while (d && done < sh->count) {
+        const int a = sh->first + done;
+        int m = 0, rc;
+        long long px = 0;
+        while (done + m < sh->count && m < CHUNK_PICTURES && (m == 0 || px + (long long)sh->ysz[a + m] * sh->xsz[a + m] <= CHUNK_PIXELS))
+            px += (long long)sh->ysz[a + m] * sh->xsz[a + m], m++;
+        rc = hevce_decoder_upload(d, m, sh->streams + a, sh->stream_len + a);
+        if (!rc) rc = hevce_decoder_run(d);
+        if (rc) { sh->status = rc; break; }
+        rc = hevce_decoder_download(d, sh->decs + a, sh->pic_status ? sh->pic_status + a : NULL);
+        done += m;
+        if (rc == HEVCE_ERR_STATE) sh->status = rc;   /* pictures that did not parse: the next chunks still run */
+        else if (rc) { sh->status = rc; break; }
+    }
+    if (cached) {
+        pthread_mutex_lock(&g_lock);
+        g_dec_busy[sh->device] = 0;
+        pthread_mutex_unlock(&g_lock);
+    } else if (d) {
+        hevce_decoder_destroy(d);
+    }
+    return NULL;
+}
+
+API int HEVCImageDecoderBatch(int n, const unsigned char *const *streams, const int *stream_len, unsigned char *const *img_decs, int *status) {
+    DecShard shards[MAX_DEV];
+    pthread_t threads[MAX_DEV];
+    int ndev, devs[MAX_DEV], cut_dev[MAX_DEV], cut_first[MAX_DEV], cut_count[MAX_DEV], started[MAX_DEV], *ys, *xs, i, k, q, nshard, rc = 0,
+        saved_device;
+    if (!hevce_stream_info || !hevce_decoder_create || !hevce_decoder_upload || !hevce_decoder_run || !hevce_decoder_download ||
+        !hevce_decoder_destroy)
+        return HEVCE_ERR_STATE;   /* linked without the decoder */
+    if (n < 0) return HEVCE_ERR_ARG;
+    if (n == 0) return 0;
+    if (!streams || !stream_len || !img_decs) return HEVCE_ERR_ARG;
+    ys = (int *)malloc(sizeof(int) * (size_t)n);
+    xs = (int *)malloc(sizeof(int) * (size_t)n);
+    for (i = 0; ys && xs && i < n && !rc; i++)
+        if (!streams[i] || !img_decs[i] || hevce_stream_info(streams[i], stream_len[i], &ys[i], &xs[i], &q)) rc = HEVCE_ERR_ARG;
+    if (!ys || !xs) rc = HEVCE_ERR_ARG;
+    if (!rc) {
+        pthread_mutex_lock(&g_lock);
+        ndev = resolve_devices();
+        if (ndev > 0) memcpy(devs, g_devs, sizeof(int) * (size_t)ndev);
+        pthread_mutex_unlock(&g_lock);
+        if (ndev < 0) rc = ndev;
+        else if (ndev == 0) {
+            fprintf(stderr, "libhevce_b200: no usable CUDA device (this library has no CPU path)\n");
+            rc = HEVCE_ERR_CUDA;
+        }
+    }
+    if (rc) { free(ys); free(xs); return rc; }
+    saved_device = hevce_internal_get_device();   /* shard 0 runs on this thread and selects its device */
+    nshard = cut_shards(n, ys, xs, 16384, ndev, devs, cut_dev, cut_first, cut_count);   /* stream sizes are padded already */
+    for (k = 0; k < nshard; k++) {
+        shards[k].device = cut_dev[k]; shards[k].first = cut_first[k]; shards[k].count = cut_count[k];
+        shards[k].streams = streams; shards[k].stream_len = stream_len; shards[k].ysz = ys; shards[k].xsz = xs;
+        shards[k].decs = img_decs; shards[k].pic_status = status;
+    }
+    for (k = 1; k < nshard; k++) {
+        started[k] = pthread_create(&threads[k], NULL, dec_shard_main, &shards[k]) == 0;
+        if (!started[k]) dec_shard_main(&shards[k]);
+    }
+    dec_shard_main(&shards[0]);
+    for (k = 1; k < nshard; k++)
+        if (started[k]) pthread_join(threads[k], NULL);
+    for (k = 0; k < nshard; k++)   /* a failed call outranks pictures that did not parse */
+        if (shards[k].status && (!rc || rc == HEVCE_ERR_STATE)) rc = shards[k].status;
+    free(ys);
+    free(xs);
+    hevce_internal_set_device(saved_device);   /* leave the caller's current device as it was */
+    return rc;
 }

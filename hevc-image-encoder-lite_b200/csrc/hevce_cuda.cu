@@ -23,6 +23,7 @@
 #include "../../include/hevce.h"
 #include "hevce_core.h"
 #include "hevce_deblock.h"
+#include "hevce_decode.h"
 #include "hevce_internal.h"
 #include "hevce_variants.h"
 
@@ -115,6 +116,75 @@ __global__ void __launch_bounds__(DBK_THREADS) hevce_deblock_kernel(const Job* _
     }
     u8* dec = dec_base + (job.rcon - rcon_base);
     for (int i = threadIdx.x; i < DBK_STORE_ITEMS; i += DBK_THREADS) dbk_store(t, job, ctu, dec, i);
+}
+
+// f6, the decoder (hevce_decode.h).  A picture's stream: its bytes, header length (first byte of the slice data), length.
+struct DecSrc { const u8* data; int start, len; };
+
+// Parse: the CABAC state threads through a picture's whole slice, so one lane of a warp parses one picture (blockIdx.x).
+// Fills the picture's CtuRec partition bytes and its (zeroed) level blocks; status[picture] = DEC_OK or DEC_ERR.
+__global__ void __launch_bounds__(32) hevce_parse_kernel(const Job* __restrict__ jobs, const DecSrc* __restrict__ src,
+                                                         const Tables* __restrict__ tables, int* __restrict__ status) {
+    __shared__ Tables tb;
+    for (int i = threadIdx.x; i < (int)(sizeof(Tables) / 4); i += 32) ((u32*)&tb)[i] = ((const u32*)tables)[i];
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        const DecSrc s = src[blockIdx.x];
+        status[blockIdx.x] = dec_parse_picture(jobs[blockIdx.x], s.data, s.start, s.len, tb);
+    }
+}
+
+// Reconstruction: one CTA per picture (blockIdx.x), a CTU-row wavefront.  Warp w takes CTU rows w, w + DEC_WARPS, ...; it
+// starts CTU (r, c) once row r - 1 has finished CTU c + 1 (the above-right samples), and the lanes of the warp share the
+// phases of each TU (reference samples, filtering: one sample each; columns, then rows of the inverse transform and the
+// prediction: one line each).  A picture whose parse failed is written as zeros.
+constexpr int DEC_WARPS = 8;
+struct DecWarp { DecTuWork w; DecTu tus[64]; int nt; };
+
+__global__ void __launch_bounds__(32 * DEC_WARPS) hevce_recon_kernel(const Job* __restrict__ jobs, const int* __restrict__ status) {
+    __shared__ DecWarp ws[DEC_WARPS];
+    __shared__ int done[DEC_MAX_DIM / CTU];   // CTUs finished per CTU row
+    const Job job = jobs[blockIdx.x];
+    const int rows = job.H / CTU, cols = job.W / CTU;
+    if (status[blockIdx.x] != DEC_OK) {
+        for (size_t i = threadIdx.x; i < (size_t)job.H * job.W / 16; i += blockDim.x) ((uint4*)job.rcon)[i] = make_uint4(0, 0, 0, 0);
+        return;
+    }
+    for (int i = threadIdx.x; i < rows; i += blockDim.x) done[i] = 0;
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    DecWarp& s = ws[threadIdx.x >> 5];
+    volatile int* vdone = done;
+    for (int r = threadIdx.x >> 5; r < rows; r += DEC_WARPS) {
+        for (int c = 0; c < cols; c++) {
+            if (r > 0 && lane == 0) {
+                const int need = min(c + 2, cols);
+                while (vdone[r - 1] < need) __nanosleep(32);
+                __threadfence_block();
+            }
+            const int ctu = r * cols + c;
+            if (lane == 0) s.nt = dec_tu_list(job.recs[ctu], s.tus);
+            __syncwarp();
+            const s16* lev = job.levs + (size_t)ctu * (CTU * CTU);
+            for (int t = 0; t < s.nt; t++) {
+                const DecTu u = s.tus[t];
+                const int T = u.s, ty = r * CTU + u.y, tx = c * CTU + u.x;
+                for (int j = lane; j < dec_ref_items(T); j += 32) dec_ref_item(s.w, job, ty, tx, T, j);
+                __syncwarp();
+                if (lane == 0) dec_ref_substitute(s.w, T);
+                __syncwarp();
+                for (int j = lane; j < dec_ref_items(T); j += 32) dec_filter_item(s.w, T, j);
+                if (lane < T) dec_column(s.w, lev + u.y * CTU + u.x, T, job.q, lane);
+                __syncwarp();
+                if (lane < T) dec_row(s.w, job, ty, tx, T, u.m, lane);
+                __syncwarp();
+            }
+            if (lane == 0) {
+                __threadfence_block();
+                vdone[r] = c + 1;
+            }
+        }
+    }
 }
 
 // integer-issue micro-benchmark: 8 independent IMAD chains + 8 independent LOP3/IADD3 chains per thread
@@ -661,6 +731,171 @@ extern "C" void hevce_session_destroy(hevce_session* s) {
     if (s->stream) cudaStreamDestroy(s->stream);
     delete s;
 }
+
+// ------------------------------------------------------------------------------------------------------------
+// f6: the decoder -- streams of this library back to decoded pictures, separate from the encoder's sessions
+// ------------------------------------------------------------------------------------------------------------
+extern "C" int hevce_stream_info(const unsigned char* stream, int len, int* ysz, int* xsz, int* qpd6) {
+    int H, W, q;
+    if (!stream || len <= 0 || dec_header(stream, len, H, W, q) < 0) return HEVCE_ERR_ARG;
+    if (ysz) *ysz = H;
+    if (xsz) *xsz = W;
+    if (qpd6) *qpd6 = q;
+    return 0;
+}
+
+struct hevce_decoder {
+    int device = 0, n = 0, max_nctu = 0;
+    bool ran = false;                 // hevce_decoder_run has run since the last upload
+    float parse_ms = 0.f, recon_ms = 0.f, deblock_ms = 0.f;
+    cudaStream_t stream = nullptr;
+    cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
+    std::vector<Job> jobs;
+    std::vector<DecSrc> src;
+    std::vector<size_t> pix_off;
+    std::vector<int> status;
+    size_t pix_total = 0;
+    GrowBuffer<u8> d_bits, d_rcon, d_dec;
+    GrowBuffer<Job> d_jobs;
+    GrowBuffer<DecSrc> d_src;
+    GrowBuffer<int> d_status;
+    GrowBuffer<CtuRec> d_recs;
+    GrowBuffer<s16> d_levs;
+    GrowBuffer<u8, true> h_stage;     // pinned staging
+};
+
+extern "C" void hevce_decoder_destroy(hevce_decoder* d) {
+    if (!d) return;
+    cudaSetDevice(d->device);
+    for (cudaEvent_t e : d->ev) if (e) cudaEventDestroy(e);
+    if (d->stream) cudaStreamDestroy(d->stream);
+    delete d;
+}
+
+extern "C" hevce_decoder* hevce_decoder_create(int device) {
+    if (device_prepare(device)) return nullptr;
+    hevce_decoder* d = new hevce_decoder;
+    d->device = device;
+    bool ok = cudaStreamCreateWithFlags(&d->stream, cudaStreamNonBlocking) == cudaSuccess;
+    for (cudaEvent_t& e : d->ev) ok = ok && cudaEventCreate(&e) == cudaSuccess;
+    if (!ok) {
+        fprintf(stderr, "libhevce_b200: cannot create stream/events on device %d\n", device);
+        hevce_decoder_destroy(d);
+        return nullptr;
+    }
+    return d;
+}
+
+// n streams -> device: every header is checked first (HEVCE_ERR_ARG, nothing changed), then the streams go up as one copy
+extern "C" int hevce_decoder_upload(hevce_decoder* d, int n, const unsigned char* const* streams, const int* stream_len) {
+    if (!d || n < 0 || n > 65535 || (n > 0 && (!streams || !stream_len))) return HEVCE_ERR_ARG;   // grid.y of the deblocking kernel
+    std::vector<Job> jobs((size_t)n);
+    std::vector<DecSrc> src((size_t)n);
+    std::vector<size_t> pix_off((size_t)n), bit_off((size_t)n), ctu_off((size_t)n);
+    size_t pix = 0, bits = 0, ctus = 0;
+    int max_nctu = 0;
+    for (int i = 0; i < n; i++) {
+        Job& j = jobs[i];
+        memset(&j, 0, sizeof(Job));
+        if (!streams[i] || stream_len[i] <= 0 || (src[i].start = dec_header(streams[i], stream_len[i], j.H, j.W, j.q)) < 0) return HEVCE_ERR_ARG;
+        src[i].len = stream_len[i];
+        j.src_h = j.H; j.src_w = j.W;
+        pix_off[i] = pix; bit_off[i] = bits; ctu_off[i] = ctus;
+        pix += (size_t)j.H * j.W;
+        bits += ((size_t)stream_len[i] + 15) & ~(size_t)15;
+        ctus += (size_t)(j.H / CTU) * (j.W / CTU);
+        max_nctu = std::max(max_nctu, (j.H / CTU) * (j.W / CTU));
+    }
+    CK(cudaSetDevice(d->device));
+    d->ran = false;
+    d->n = n;
+    if (n == 0) return 0;
+    int rc;
+    if ((rc = d->h_stage.reserve(bits))) return rc;
+    if ((rc = d->d_bits.reserve(bits))) return rc;
+    if ((rc = d->d_rcon.reserve(pix))) return rc;
+    if ((rc = d->d_dec.reserve(pix))) return rc;
+    if ((rc = d->d_jobs.reserve((size_t)n))) return rc;
+    if ((rc = d->d_src.reserve((size_t)n))) return rc;
+    if ((rc = d->d_status.reserve((size_t)n))) return rc;
+    if ((rc = d->d_recs.reserve(ctus))) return rc;
+    if ((rc = d->d_levs.reserve(ctus * CTU * CTU))) return rc;
+    parallel_pictures(n, bits, [&](int i) { memcpy(d->h_stage.p + bit_off[i], streams[i], (size_t)stream_len[i]); });
+    for (int i = 0; i < n; i++) {
+        jobs[i].rcon = d->d_rcon.p + pix_off[i];
+        jobs[i].recs = d->d_recs.p + ctu_off[i];
+        jobs[i].levs = d->d_levs.p + ctu_off[i] * CTU * CTU;
+        src[i].data = d->d_bits.p + bit_off[i];
+    }
+    CK(cudaMemcpyAsync(d->d_bits.p, d->h_stage.p, bits, cudaMemcpyHostToDevice, d->stream));
+    CK(cudaMemcpyAsync(d->d_jobs.p, jobs.data(), (size_t)n * sizeof(Job), cudaMemcpyHostToDevice, d->stream));
+    CK(cudaMemcpyAsync(d->d_src.p, src.data(), (size_t)n * sizeof(DecSrc), cudaMemcpyHostToDevice, d->stream));
+    CK(cudaStreamSynchronize(d->stream));
+    d->jobs.swap(jobs);
+    d->src.swap(src);
+    d->pix_off.swap(pix_off);
+    d->pix_total = pix;
+    d->max_nctu = max_nctu;
+    return 0;
+}
+
+// parse + reconstruction + deblocking of the uploaded streams, synchronous
+extern "C" int hevce_decoder_run(hevce_decoder* d) {
+    if (!d) return HEVCE_ERR_ARG;
+    CK(cudaSetDevice(d->device));
+    if (d->n > 0) {
+        size_t ctus = 0;
+        for (const Job& j : d->jobs) ctus += (size_t)(j.H / CTU) * (j.W / CTU);
+        CK(cudaMemsetAsync(d->d_levs.p, 0, ctus * CTU * CTU * sizeof(s16), d->stream));   // the parser writes non-zero levels only
+        CK(cudaEventRecord(d->ev[0], d->stream));
+        hevce_parse_kernel<<<d->n, 32, 0, d->stream>>>(d->d_jobs.p, d->d_src.p, g_dev[d->device].d_tables, d->d_status.p);
+        CK(cudaGetLastError());
+        CK(cudaEventRecord(d->ev[1], d->stream));
+        hevce_recon_kernel<<<d->n, 32 * DEC_WARPS, 0, d->stream>>>(d->d_jobs.p, d->d_status.p);
+        CK(cudaGetLastError());
+        CK(cudaEventRecord(d->ev[2], d->stream));
+        hevce_deblock_kernel<<<dim3((unsigned)d->max_nctu, (unsigned)d->n), DBK_THREADS, 0, d->stream>>>(d->d_jobs.p, d->d_rcon.p, d->d_dec.p);
+        CK(cudaGetLastError());
+        CK(cudaEventRecord(d->ev[3], d->stream));
+        CK(cudaStreamSynchronize(d->stream));
+        CK(cudaEventElapsedTime(&d->parse_ms, d->ev[0], d->ev[1]));
+        CK(cudaEventElapsedTime(&d->recon_ms, d->ev[1], d->ev[2]));
+        CK(cudaEventElapsedTime(&d->deblock_ms, d->ev[2], d->ev[3]));
+    }
+    d->ran = true;
+    return 0;
+}
+
+// decoded pictures -> host (one copy); status[i] (may be NULL) = 0 or HEVCE_ERR_STATE.  Returns HEVCE_ERR_STATE when a
+// picture's slice data did not parse (its buffer then holds zeros); the other pictures are decoded all the same.
+extern "C" int hevce_decoder_download(hevce_decoder* d, unsigned char* const* img_decs, int* status) {
+    if (!d || (d->n > 0 && !img_decs)) return HEVCE_ERR_ARG;
+    if (d->n > 0 && !d->ran) return HEVCE_ERR_STATE;
+    CK(cudaSetDevice(d->device));
+    if (d->n == 0) return 0;
+    for (int i = 0; i < d->n; i++)
+        if (!img_decs[i]) return HEVCE_ERR_ARG;
+    int rc = d->h_stage.reserve(d->pix_total);
+    if (rc) return rc;
+    d->status.resize((size_t)d->n);
+    CK(cudaMemcpyAsync(d->status.data(), d->d_status.p, (size_t)d->n * sizeof(int), cudaMemcpyDeviceToHost, d->stream));
+    CK(cudaMemcpyAsync(d->h_stage.p, d->d_dec.p, d->pix_total, cudaMemcpyDeviceToHost, d->stream));
+    CK(cudaStreamSynchronize(d->stream));
+    parallel_pictures(d->n, d->pix_total, [&](int i) {
+        const Job& j = d->jobs[i];
+        memcpy(img_decs[i], d->h_stage.p + d->pix_off[i], (size_t)j.H * j.W);
+    });
+    int ret = 0;
+    for (int i = 0; i < d->n; i++) {
+        if (status) status[i] = d->status[i] == DEC_OK ? 0 : HEVCE_ERR_STATE;
+        if (d->status[i] != DEC_OK) ret = HEVCE_ERR_STATE;
+    }
+    return ret;
+}
+
+extern "C" float hevce_decoder_parse_ms(const hevce_decoder* d) { return d ? d->parse_ms : 0.f; }
+extern "C" float hevce_decoder_recon_ms(const hevce_decoder* d) { return d ? d->recon_ms : 0.f; }
+extern "C" float hevce_decoder_deblock_ms(const hevce_decoder* d) { return d ? d->deblock_ms : 0.f; }
 
 #if defined(HEVCE_PROFILE_DUMP)
 extern "C" __attribute__((visibility("default"))) void hevce_profile_dump(void) {

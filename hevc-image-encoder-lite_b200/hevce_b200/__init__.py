@@ -28,6 +28,8 @@ EXPORTS = [
     "hevce_set_variant", "hevce_session_variant", "hevce_get_max_dim", "hevce_release",
     "HEVCImageEncoderBatchDecoded", "hevce_session_deblock", "hevce_session_deblock_ms", "hevce_session_download_decoded",
     "hevce_session_decoded_quality",
+    "hevce_stream_info", "HEVCImageDecoderBatch", "hevce_decoder_create", "hevce_decoder_upload", "hevce_decoder_run",
+    "hevce_decoder_download", "hevce_decoder_parse_ms", "hevce_decoder_recon_ms", "hevce_decoder_deblock_ms", "hevce_decoder_destroy",
 ]
 
 
@@ -98,6 +100,23 @@ def lib():
             getattr(L, f).argtypes = [ctypes.c_void_p]
         L.hevce_session_destroy.restype = None
         L.hevce_session_destroy.argtypes = [ctypes.c_void_p]
+        L.hevce_stream_info.restype = ctypes.c_int
+        L.hevce_stream_info.argtypes = [_u8p, ctypes.c_int, _ip, _ip, _ip]
+        L.HEVCImageDecoderBatch.restype = ctypes.c_int
+        L.HEVCImageDecoderBatch.argtypes = [ctypes.c_int, ctypes.POINTER(_u8p), _ip, ctypes.POINTER(_u8p), _ip]
+        L.hevce_decoder_create.restype = ctypes.c_void_p
+        L.hevce_decoder_create.argtypes = [ctypes.c_int]
+        L.hevce_decoder_upload.restype = ctypes.c_int
+        L.hevce_decoder_upload.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(_u8p), _ip]
+        L.hevce_decoder_run.restype = ctypes.c_int
+        L.hevce_decoder_run.argtypes = [ctypes.c_void_p]
+        L.hevce_decoder_download.restype = ctypes.c_int
+        L.hevce_decoder_download.argtypes = [ctypes.c_void_p, ctypes.POINTER(_u8p), _ip]
+        for f in ("hevce_decoder_parse_ms", "hevce_decoder_recon_ms", "hevce_decoder_deblock_ms"):
+            getattr(L, f).restype = ctypes.c_float
+            getattr(L, f).argtypes = [ctypes.c_void_p]
+        L.hevce_decoder_destroy.restype = None
+        L.hevce_decoder_destroy.argtypes = [ctypes.c_void_p]
         _lib = L
     return _lib
 
@@ -337,6 +356,97 @@ class Session:
     def close(self):
         if self._h:
             lib().hevce_session_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+# ---- f6: decoding the streams this library writes --------------------------------------------------------------
+def _streams(streams):
+    arrs = [np.frombuffer(bytes(s), np.uint8).copy() for s in streams]
+    return arrs, (ctypes.c_int * len(arrs))(*[a.size for a in arrs])
+
+
+def stream_info(stream):
+    """(ysz, xsz, qpd6) of a stream this library wrote: its padded size and qpd6.  A header check on the host, no device.
+    Raises HevceError(ERR_ARG) for a stream whose parameter sets are not the ones this library writes."""
+    a = np.frombuffer(bytes(stream), np.uint8).copy()
+    y, x, q = ctypes.c_int(), ctypes.c_int(), ctypes.c_int()
+    rc = lib().hevce_stream_info(a.ctypes.data_as(_u8p), int(a.size), ctypes.byref(y), ctypes.byref(x), ctypes.byref(q))
+    if rc < 0:
+        raise HevceError(rc, "hevce_stream_info")
+    return y.value, x.value, q.value
+
+
+def HEVCImageDecoderBatch(streams, return_status=False):
+    """Decode streams of this library on the device: the decoded pictures at their padded size (what
+    HEVCImageEncoderBatchDecoded returns as decoded).  A stream whose slice data does not parse raises HevceError(ERR_STATE),
+    unless return_status: then (pictures, status) is returned, status[i] 0 or ERR_STATE (that picture is all zeros)."""
+    arrs, lens = _streams(streams)
+    n = len(arrs)
+    decs = []
+    for a in arrs:
+        y, x, _ = stream_info(a)
+        decs.append(np.zeros((y, x), np.uint8))
+    st = (ctypes.c_int * n)()
+    rc = lib().HEVCImageDecoderBatch(n, _ptr_array(arrs), lens, _ptr_array(decs), st)
+    if rc < 0 and not (return_status and rc == ERR_STATE):
+        raise HevceError(rc, "HEVCImageDecoderBatch")
+    return (decs, list(st)) if return_status else decs
+
+
+class Decoder:
+    """Device-resident decoder on one GPU: upload streams, run the parse / reconstruction / deblocking kernels (timed with
+    CUDA events), download the decoded pictures."""
+
+    def __init__(self, device=0):
+        self._h = lib().hevce_decoder_create(int(device))
+        if not self._h:
+            raise HevceError(ERR_CUDA, "hevce_decoder_create")
+        self.shapes = []
+
+    def upload(self, streams):
+        arrs, lens = _streams(streams)
+        shapes = [stream_info(a)[:2] for a in arrs]
+        rc = lib().hevce_decoder_upload(self._h, len(arrs), _ptr_array(arrs), lens)
+        if rc < 0:
+            raise HevceError(rc, "hevce_decoder_upload")
+        self.shapes = shapes
+
+    def run(self):
+        """Decode the uploaded streams (synchronous); returns the three kernels' total ms."""
+        rc = lib().hevce_decoder_run(self._h)
+        if rc < 0:
+            raise HevceError(rc, "hevce_decoder_run")
+        return self.parse_ms + self.recon_ms + self.deblock_ms
+
+    def download(self, return_status=False):
+        decs = [np.zeros(s, np.uint8) for s in self.shapes]
+        st = (ctypes.c_int * max(1, len(decs)))()
+        rc = lib().hevce_decoder_download(self._h, _ptr_array(decs), st)
+        if rc < 0 and not (return_status and rc == ERR_STATE):
+            raise HevceError(rc, "hevce_decoder_download")
+        return (decs, list(st)[:len(decs)]) if return_status else decs
+
+    @property
+    def parse_ms(self):
+        return lib().hevce_decoder_parse_ms(self._h)
+
+    @property
+    def recon_ms(self):
+        return lib().hevce_decoder_recon_ms(self._h)
+
+    @property
+    def deblock_ms(self):
+        return lib().hevce_decoder_deblock_ms(self._h)
+
+    def close(self):
+        if self._h:
+            lib().hevce_decoder_destroy(self._h)
             self._h = None
 
     def __del__(self):

@@ -127,6 +127,37 @@ HEVCE_API long long hevce_session_h2d_bytes(const hevce_session *s);
 HEVCE_API long long hevce_session_d2h_bytes(const hevce_session *s);
 HEVCE_API void hevce_session_destroy(hevce_session *s);
 
+/* ---- f6: decoding the streams this library writes ------------------------------------------------------------
+ * The decoder accepts exactly the parameter sets and slice header this library writes (one I slice, luma only, CTB 32,
+ * no SAO, deblocking on; write_header in csrc/hevce_core.h) and returns the decoded picture at the padded size the stream
+ * carries, stride = padded width: for a stream of HEVCImageEncoderBatchDecoded, its img_decs.  Any other stream is
+ * rejected by the header check, not decoded.  Decoding runs on the device only (HEVCE_ERR_CUDA without one). */
+
+/* Padded size and qpd6 of a stream this library wrote.  Host-only header check, needs no device.  Returns 0, or
+ * HEVCE_ERR_ARG if the parameter sets and slice header are not the ones this library writes.  Any output may be NULL. */
+HEVCE_API int hevce_stream_info(const unsigned char *stream, int len, int *ysz, int *xsz, int *qpd6);
+
+/* n streams -> n decoded pictures; img_decs[i] holds ysz * xsz bytes of hevce_stream_info.  status[i] (may be NULL)
+ * receives 0, or HEVCE_ERR_STATE when the slice data of stream i does not parse (its picture is then all zeros; the
+ * other pictures are decoded all the same and the call returns HEVCE_ERR_STATE).  Sharded over the selected devices like
+ * HEVCImageEncoderBatch.  HEVCE_ERR_ARG, before any device work, if any header is rejected.  The caller's current
+ * device is restored. */
+HEVCE_API int HEVCImageDecoderBatch(int n, const unsigned char *const *streams, const int *stream_len,
+                          unsigned char *const *img_decs, int *status);
+
+/* Device-resident decoder on ONE device, independent of the encoder's sessions. */
+typedef struct hevce_decoder hevce_decoder;
+HEVCE_API hevce_decoder *hevce_decoder_create(int device);
+/* host -> HBM, one packed copy; HEVCE_ERR_ARG (nothing uploaded) if a header is rejected */
+HEVCE_API int   hevce_decoder_upload(hevce_decoder *d, int n, const unsigned char *const *streams, const int *stream_len);
+HEVCE_API int   hevce_decoder_run(hevce_decoder *d);   /* parse + reconstruction + deblocking kernels, synchronous */
+/* HBM -> host; status as for HEVCImageDecoderBatch; HEVCE_ERR_STATE before hevce_decoder_run or if a picture failed */
+HEVCE_API int   hevce_decoder_download(hevce_decoder *d, unsigned char *const *img_decs, int *status);
+HEVCE_API float hevce_decoder_parse_ms(const hevce_decoder *d);     /* CUDA-event durations of the three kernels of */
+HEVCE_API float hevce_decoder_recon_ms(const hevce_decoder *d);     /* the last hevce_decoder_run                   */
+HEVCE_API float hevce_decoder_deblock_ms(const hevce_decoder *d);
+HEVCE_API void  hevce_decoder_destroy(hevce_decoder *d);
+
 /* Integer-issue peak of the device: a dependency-free IMAD/LOP3 micro-benchmark; returns int-ops/s (IMAD = 2 ops),
  * or a negative HEVCE_ERR_*.  Used as the roofline denominator companion (SURVEY.md section 8d). */
 HEVCE_API double hevce_measure_int_peak(int device);
