@@ -5,6 +5,7 @@
  *   HEVCImageEncoderBatch  n independent pictures, sharded over the selected GPUs by cumulative CTU count,
  *                          no collective (SURVEY.md section 8e)
  *   HEVCImageEncoderBatchDecoded  the same, plus every picture after the in-loop deblocking filter
+ *   HEVCImageEncoderBatchTarget   each picture at the coarsest qpd6 whose decoded picture meets a quality target
  *   HEVCImageDecoderBatch  streams of this library back to decoded pictures, sharded the same way
  *
  * A shard (the pictures of one device) is cut into chunks; same-size pictures run as rounds of four chunks on four host
@@ -15,6 +16,7 @@
  * used the calls fail with HEVCE_ERR_CUDA.
  */
 #include <errno.h>
+#include <math.h>
 #include <pthread.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -28,6 +30,9 @@
    define them, such as the CPU stand-in of the chunk-planner test; in libhevce_b200.so hevce_cuda.cu defines both. */
 #pragma weak hevce_session_deblock
 #pragma weak hevce_session_download_decoded
+/* ... and only HEVCImageEncoderBatchTarget these two (it returns HEVCE_ERR_STATE without the ones its metric needs). */
+#pragma weak hevce_session_ssim
+#pragma weak hevce_session_decoded_quality
 /* The same for the decoder (HEVCImageDecoderBatch returns HEVCE_ERR_STATE without them). */
 #pragma weak hevce_stream_info
 #pragma weak hevce_decoder_create
@@ -166,6 +171,8 @@ typedef struct {
     unsigned char *const *decs;   /* decoded pictures, or NULL: HEVCImageEncoderBatch */
     const int *ysz, *xsz, *qpd6;
     int *stream_len;
+    int metric;                   /* HEVCE_METRIC_* of quality */
+    double *quality;              /* decoded pictures' quality, or NULL: only HEVCImageEncoderBatchTarget asks for it */
     /* chunk queue shared by the shard's workers */
     int nchunk, next_chunk;
     int *chunk_first;   /* nchunk + 1 entries; a chunk holds at least one picture, so count + 1 are allocated */
@@ -200,7 +207,9 @@ static void *chunk_worker(void *arg) {
         if (!rc) rc = hevce_session_upload(s, sh->imgs + a);
         if (!rc) rc = hevce_session_encode(s);
         if (!rc) rc = hevce_session_download(s, sh->pbuffers + a, sh->rcons + a, sh->stream_len + a);
-        if (!rc && sh->decs) rc = hevce_session_deblock(s);
+        if (!rc && (sh->decs || sh->quality)) rc = hevce_session_deblock(s);
+        if (!rc && sh->quality)
+            rc = sh->metric == HEVCE_METRIC_SSIM ? hevce_session_ssim(s, 1, sh->quality + a) : hevce_session_decoded_quality(s, NULL, sh->quality + a);
         if (!rc && sh->decs) rc = hevce_session_download_decoded(s, sh->decs + a);
         if (rc) {
             pthread_mutex_lock(&sh->qlock);
@@ -296,14 +305,24 @@ static int cut_shards(int n, const int *ysz, const int *xsz, int max_dim, int nd
     return nshard;
 }
 
-/* both batch entry points; img_decs NULL: no decoded pictures */
+/* size write-back (HEVCe.c:1643-1644) */
+static void write_sizes(int n, int *ysz, int *xsz, int max_dim) {
+    int i;
+    for (i = 0; i < n; i++) {
+        ysz[i] = padded_dim(ysz[i], max_dim);
+        xsz[i] = padded_dim(xsz[i], max_dim);
+    }
+}
+
+/* the batch path of every encoding entry point; img_decs NULL: no decoded pictures; quality NULL: no quality reduction.
+   max_dim is the caller's one value for the whole call (sharding, clamp and size write-back); the sizes are not written. */
 static int encode_batch(int n, unsigned char *const *pbuffers, const unsigned char *const *imgs, unsigned char *const *img_rcons,
-                        unsigned char *const *img_decs, int *ysz, int *xsz, const int *qpd6, int *stream_len) {
+                        unsigned char *const *img_decs, const int *ysz, const int *xsz, const int *qpd6, int *stream_len, int max_dim,
+                        int metric, double *quality) {
     Shard shards[MAX_DEV];
     pthread_t threads[MAX_DEV];
     int ndev, devs[MAX_DEV], started[MAX_DEV], i, k, nshard = 0, status = 0, *lens = stream_len, saved_device;
     int cut_dev[MAX_DEV], cut_first[MAX_DEV], cut_count[MAX_DEV];
-    const int max_dim = hevce_get_max_dim();   /* one value for the whole call: sharding, clamp and size write-back */
     if (n < 0) return HEVCE_ERR_ARG;
     if (n == 0) return 0;
     if (!pbuffers || !imgs || !img_rcons || !ysz || !xsz || !qpd6) return HEVCE_ERR_ARG;
@@ -326,6 +345,7 @@ static int encode_batch(int n, unsigned char *const *pbuffers, const unsigned ch
         shards[k].device = cut_dev[k]; shards[k].first = cut_first[k]; shards[k].count = cut_count[k]; shards[k].max_dim = max_dim;
         shards[k].pbuffers = pbuffers; shards[k].imgs = imgs; shards[k].rcons = img_rcons; shards[k].decs = img_decs;
         shards[k].ysz = ysz; shards[k].xsz = xsz; shards[k].qpd6 = qpd6; shards[k].stream_len = lens;
+        shards[k].metric = metric; shards[k].quality = quality;
     }
     for (k = 1; k < nshard; k++) {
         started[k] = pthread_create(&threads[k], NULL, shard_main, &shards[k]) == 0;
@@ -336,11 +356,6 @@ static int encode_batch(int n, unsigned char *const *pbuffers, const unsigned ch
         if (started[k]) pthread_join(threads[k], NULL);
     for (k = 0; k < nshard; k++)
         if (shards[k].status && !status) status = shards[k].status;
-    if (!status)
-        for (i = 0; i < n; i++) {   /* size write-back (HEVCe.c:1643-1644) */
-            ysz[i] = padded_dim(ysz[i], max_dim);
-            xsz[i] = padded_dim(xsz[i], max_dim);
-        }
     if (lens != stream_len) free(lens);
     hevce_internal_set_device(saved_device);      /* leave the caller's current device as it was */
     return status;
@@ -348,17 +363,109 @@ static int encode_batch(int n, unsigned char *const *pbuffers, const unsigned ch
 
 API int HEVCImageEncoderBatch(int n, unsigned char *const *pbuffers, const unsigned char *const *imgs,
                               unsigned char *const *img_rcons, int *ysz, int *xsz, const int *qpd6, int *stream_len) {
-    return encode_batch(n, pbuffers, imgs, img_rcons, NULL, ysz, xsz, qpd6, stream_len);
+    const int max_dim = hevce_get_max_dim();
+    const int rc = encode_batch(n, pbuffers, imgs, img_rcons, NULL, ysz, xsz, qpd6, stream_len, max_dim, 0, NULL);
+    if (!rc) write_sizes(n, ysz, xsz, max_dim);
+    return rc;
 }
 
 API int HEVCImageEncoderBatchDecoded(int n, unsigned char *const *pbuffers, const unsigned char *const *imgs, unsigned char *const *img_rcons,
                                      unsigned char *const *img_decs, int *ysz, int *xsz, const int *qpd6, int *stream_len) {
-    int i;
+    const int max_dim = hevce_get_max_dim();
+    int i, rc;
     if (!hevce_session_deblock || !hevce_session_download_decoded) return HEVCE_ERR_STATE;   /* linked without them */
     if (n > 0 && !img_decs) return HEVCE_ERR_ARG;
     for (i = 0; i < n; i++)
         if (!img_decs[i]) return HEVCE_ERR_ARG;
-    return encode_batch(n, pbuffers, imgs, img_rcons, img_decs, ysz, xsz, qpd6, stream_len);
+    rc = encode_batch(n, pbuffers, imgs, img_rcons, img_decs, ysz, xsz, qpd6, stream_len, max_dim, 0, NULL);
+    if (!rc) write_sizes(n, ysz, xsz, max_dim);
+    return rc;
+}
+
+/* Quality-target search (the rule is in hevce.h).  Each round encodes the pictures still searching, at their probe qpd6,
+   through encode_batch.  A picture without a passing probe yet encodes straight into the caller's buffers; one whose
+   buffers hold a passing probe encodes into host scratch, copied over only if the new probe passes too.  So the caller's
+   buffers always hold the last passing probe, or, while none has passed, the last probe: at the end, the chosen one. */
+API int HEVCImageEncoderBatchTarget(int n, unsigned char *const *pbuffers, const unsigned char *const *imgs, unsigned char *const *img_rcons,
+                                    unsigned char *const *img_decs, int *ysz, int *xsz, int metric, const double *target, int *qpd6,
+                                    double *quality, int *stream_len) {
+    const int max_dim = hevce_get_max_dim();
+    int i, k, m, rc = 0, *ints;
+    int *lo, *hi, *len, *idx, *sub_ys, *sub_xs, *sub_q, *sub_len;
+    double *dbls, *qual, *sub_qual;
+    unsigned char **ptrs, **sub_pb, **sub_rc, **sub_dec;
+    const unsigned char **sub_img;
+    if (metric != HEVCE_METRIC_PSNR && metric != HEVCE_METRIC_SSIM) return HEVCE_ERR_ARG;
+    if (!hevce_session_deblock || (img_decs && !hevce_session_download_decoded) ||
+        (metric == HEVCE_METRIC_SSIM ? !hevce_session_ssim : !hevce_session_decoded_quality))
+        return HEVCE_ERR_STATE;   /* linked without a call the metric needs */
+    if (n < 0) return HEVCE_ERR_ARG;
+    if (n == 0) return 0;
+    if (!pbuffers || !imgs || !img_rcons || !ysz || !xsz || !target || !qpd6) return HEVCE_ERR_ARG;
+    for (i = 0; i < n; i++)
+        if (!pbuffers[i] || !imgs[i] || !img_rcons[i] || (img_decs && !img_decs[i]) || ysz[i] <= 0 || xsz[i] <= 0 || isnan(target[i]))
+            return HEVCE_ERR_ARG;
+    ints = (int *)malloc(sizeof(int) * 8 * (size_t)n);
+    dbls = (double *)malloc(sizeof(double) * 2 * (size_t)n);
+    ptrs = (unsigned char **)malloc(sizeof(unsigned char *) * 4 * (size_t)n);
+    if (!ints || !dbls || !ptrs) {
+        free(ints); free(dbls); free(ptrs);
+        return HEVCE_ERR_ARG;
+    }
+    lo = ints; hi = lo + n; len = hi + n; idx = len + n; sub_ys = idx + n; sub_xs = sub_ys + n; sub_q = sub_xs + n; sub_len = sub_q + n;
+    qual = dbls; sub_qual = qual + n;
+    sub_pb = ptrs; sub_rc = sub_pb + n; sub_dec = sub_rc + n; sub_img = (const unsigned char **)(sub_dec + n);
+    for (i = 0; i < n; i++) lo[i] = -1, hi[i] = 5;
+    for (;;) {
+        size_t scratch_bytes = 0, off = 0;
+        unsigned char *scratch = NULL;
+        for (i = 0, m = 0; i < n; i++) {
+            if (hi[i] - lo[i] <= 1) continue;
+            idx[m] = i; sub_q[m] = (lo[i] + hi[i]) / 2; sub_ys[m] = ysz[i]; sub_xs[m] = xsz[i]; sub_img[m] = imgs[i];
+            if (lo[i] >= 0) scratch_bytes += (size_t)padded_pixels(ysz[i], xsz[i], max_dim) * (img_decs ? 4 : 3) + 256;
+            m++;
+        }
+        if (m == 0) break;
+        if (scratch_bytes && !(scratch = (unsigned char *)malloc(scratch_bytes))) { rc = HEVCE_ERR_ARG; break; }
+        for (k = 0; k < m; k++) {
+            i = idx[k];
+            if (lo[i] < 0) {
+                sub_pb[k] = pbuffers[i]; sub_rc[k] = img_rcons[i]; sub_dec[k] = img_decs ? img_decs[i] : NULL;
+            } else {   /* stream (256 + 2 B/pixel), reconstruction, decoded picture */
+                const size_t px = (size_t)padded_pixels(ysz[i], xsz[i], max_dim);
+                sub_pb[k] = scratch + off; off += 256 + 2 * px;
+                sub_rc[k] = scratch + off; off += px;
+                sub_dec[k] = NULL;
+                if (img_decs) { sub_dec[k] = scratch + off; off += px; }
+            }
+        }
+        rc = encode_batch(m, sub_pb, sub_img, sub_rc, img_decs ? sub_dec : NULL, sub_ys, sub_xs, sub_q, sub_len, max_dim, metric, sub_qual);
+        for (k = 0; !rc && k < m; k++) {
+            const int pass = sub_qual[k] >= target[idx[k]], direct = lo[idx[k]] < 0;
+            i = idx[k];
+            if (pass && !direct) {   /* a better passing probe replaces the one in the caller's buffers */
+                const size_t px = (size_t)padded_pixels(ysz[i], xsz[i], max_dim);
+                memcpy(pbuffers[i], sub_pb[k], (size_t)sub_len[k]);
+                memcpy(img_rcons[i], sub_rc[k], px);
+                if (img_decs) memcpy(img_decs[i], sub_dec[k], px);
+            }
+            if (pass || direct) { len[i] = sub_len[k]; qual[i] = sub_qual[k]; }
+            if (pass) lo[i] = sub_q[k];
+            else hi[i] = sub_q[k];
+        }
+        free(scratch);
+        if (rc) break;
+    }
+    if (!rc) {
+        for (i = 0; i < n; i++) {
+            qpd6[i] = lo[i] >= 0 ? lo[i] : 0;
+            if (quality) quality[i] = qual[i];
+            if (stream_len) stream_len[i] = len[i];
+        }
+        write_sizes(n, ysz, xsz, max_dim);
+    }
+    free(ints); free(dbls); free(ptrs);
+    return rc;
 }
 
 API int HEVCImageEncoder(unsigned char *pbuffer, const unsigned char *img, unsigned char *img_rcon, int *ysz, int *xsz, const int qpd6) {

@@ -25,6 +25,7 @@
 #include "hevce_deblock.h"
 #include "hevce_decode.h"
 #include "hevce_internal.h"
+#include "hevce_ssim.h"
 #include "hevce_variants.h"
 
 using namespace hevce;
@@ -116,6 +117,38 @@ __global__ void __launch_bounds__(DBK_THREADS) hevce_deblock_kernel(const Job* _
     }
     u8* dec = dec_base + (job.rcon - rcon_base);
     for (int i = threadIdx.x; i < DBK_STORE_ITEMS; i += DBK_THREADS) dbk_store(t, job, ctu, dec, i);
+}
+
+// f7: SSIM (hevce_ssim.h).  One CTA per (32x32 block of window centres, picture), blockIdx.y = picture.  The measured
+// plane is at the picture's reconstruction offset from rcon_base in plane_base (rcon_base itself, or the decoded
+// pictures); block b's partial goes to partials[b] past the picture's first CTU record, so each picture has its own.
+__global__ void __launch_bounds__(SSIM_THREADS) hevce_ssim_kernel(const Job* __restrict__ jobs, const u8* rcon_base, const u8* plane_base,
+                                                                  const CtuRec* recs_base, double* __restrict__ partials) {
+    __shared__ SsimTile t;
+    const Job job = jobs[blockIdx.y];
+    const int blk = blockIdx.x;
+    if (blk >= ssim_nblk(job)) return;
+    const u8* plane = plane_base + (job.rcon - rcon_base);
+    for (int i = threadIdx.x; i < SSIM_LOAD_ITEMS; i += SSIM_THREADS) ssim_load(t, job, plane, blk, i);
+    __syncthreads();
+    for (int i = threadIdx.x; i < SSIM_HSUM_ITEMS; i += SSIM_THREADS) ssim_hsum(t, i);
+    __syncthreads();
+    t.red[threadIdx.x] = ssim_thread_sum(t, job, blk, threadIdx.x);
+    __syncthreads();
+    for (int half = SSIM_THREADS / 2; half > 0; half >>= 1) {
+        ssim_reduce_step(t, half, threadIdx.x);
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) partials[(job.recs - recs_base) + blk] = t.red[0];
+}
+
+// a picture's mean SSIM from its block partials, one thread per picture
+__global__ void __launch_bounds__(128) hevce_ssim_mean_kernel(const Job* __restrict__ jobs, int n, const CtuRec* recs_base,
+                                                              const double* __restrict__ partials, double* __restrict__ ssim) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const Job job = jobs[i];
+    ssim[i] = ssim_mean(job, partials + (job.recs - recs_base));
 }
 
 // f6, the decoder (hevce_decode.h).  A picture's stream: its bytes, header length (first byte of the slice data), length.
@@ -348,6 +381,8 @@ struct hevce_session {
     bool encoded = false;   // hevce_session_encode has run since the last configure/upload
     bool deblocked = false; // hevce_session_deblock has run since the last configure/upload/encode
     GrowBuffer<u8> d_dec;   // decoded pictures at the offsets of d_rcon; reserved by the first hevce_session_deblock
+    GrowBuffer<double> d_ssim_part, d_ssim;   // SSIM block partials at the CTU offsets, per-picture means
+    float ssim_ms = 0.f;
     std::vector<size_t> ctu_off;
     int line_pitch = 0;
     GrowBuffer<u8, true> h_stage;   // pinned staging
@@ -689,6 +724,32 @@ extern "C" int hevce_session_decoded_quality(hevce_session* s, double* mse, doub
     if (s->n > 0 && !s->deblocked) return HEVCE_ERR_STATE;
     return session_quality(s, true, mse, psnr);
 }
+
+// f7: per-picture mean SSIM (hevce_ssim.h) between the coded picture and the reconstruction or (decoded) the decoded
+// picture, at the padded size
+extern "C" int hevce_session_ssim(hevce_session* s, int decoded, double* ssim) {
+    if (!s || (decoded != 0 && decoded != 1) || (s->n > 0 && !ssim)) return HEVCE_ERR_ARG;
+    if (s->n > 0 && !(decoded ? s->deblocked : s->encoded)) return HEVCE_ERR_STATE;
+    CK(cudaSetDevice(s->device));
+    if (s->n == 0) return 0;
+    const Job& last = s->jobs[s->n - 1];
+    int rc = s->d_ssim_part.reserve(s->ctu_off[s->n - 1] + (size_t)ssim_nblk(last));
+    if (!rc) rc = s->d_ssim.reserve((size_t)s->n);
+    if (rc) return rc;
+    CK(cudaEventRecord(s->ev0, s->stream));
+    hevce_ssim_kernel<<<dim3((unsigned)s->max_nctu, (unsigned)s->n), SSIM_THREADS, 0, s->stream>>>(
+        s->d_jobs.p, s->d_rcon.p, decoded ? s->d_dec.p : s->d_rcon.p, s->d_recs.p, s->d_ssim_part.p);
+    CK(cudaGetLastError());
+    hevce_ssim_mean_kernel<<<(s->n + 127) / 128, 128, 0, s->stream>>>(s->d_jobs.p, s->n, s->d_recs.p, s->d_ssim_part.p, s->d_ssim.p);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(s->ev1, s->stream));
+    CK(cudaMemcpyAsync(ssim, s->d_ssim.p, (size_t)s->n * sizeof(double), cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaStreamSynchronize(s->stream));
+    CK(cudaEventElapsedTime(&s->ssim_ms, s->ev0, s->ev1));
+    s->launches += 2;
+    return 0;
+}
+extern "C" float hevce_session_ssim_ms(const hevce_session* s) { return s ? s->ssim_ms : 0.f; }
 
 // Decisions of picture i after hevce_session_encode: CU size and luma intra mode per 4x4 unit ((H/4)*(W/4) bytes each),
 // CU kind per 8x8 unit ((H/8)*(W/8) bytes: 0 one TU, 1 four TUs, 2 NxN).  Any pointer may be NULL.

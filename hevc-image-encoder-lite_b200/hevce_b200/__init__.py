@@ -15,6 +15,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(os.path.dirname(_HERE), "libhevce_b200.so")
 
 ERR_ARG, ERR_CUDA, ERR_STATE = -1, -2, -3
+METRIC_PSNR, METRIC_SSIM = 0, 1
 
 _u8p = ctypes.POINTER(ctypes.c_ubyte)
 _ip = ctypes.POINTER(ctypes.c_int)
@@ -30,6 +31,7 @@ EXPORTS = [
     "hevce_session_decoded_quality",
     "hevce_stream_info", "HEVCImageDecoderBatch", "hevce_decoder_create", "hevce_decoder_upload", "hevce_decoder_run",
     "hevce_decoder_download", "hevce_decoder_parse_ms", "hevce_decoder_recon_ms", "hevce_decoder_deblock_ms", "hevce_decoder_destroy",
+    "hevce_session_ssim", "hevce_session_ssim_ms", "HEVCImageEncoderBatchTarget",
 ]
 
 
@@ -56,6 +58,11 @@ def lib():
         L.HEVCImageEncoderBatch.argtypes = [ctypes.c_int, ctypes.POINTER(_u8p), ctypes.POINTER(_u8p), ctypes.POINTER(_u8p), _ip, _ip, _ip, _ip]
         L.HEVCImageEncoderBatchDecoded.restype = ctypes.c_int
         L.HEVCImageEncoderBatchDecoded.argtypes = [ctypes.c_int] + [ctypes.POINTER(_u8p)] * 4 + [_ip, _ip, _ip, _ip]
+        _dp = ctypes.POINTER(ctypes.c_double)
+        L.HEVCImageEncoderBatchTarget.restype = ctypes.c_int
+        L.HEVCImageEncoderBatchTarget.argtypes = [ctypes.c_int] + [ctypes.POINTER(_u8p)] * 4 + [_ip, _ip, ctypes.c_int, _dp, _ip, _dp, _ip]
+        L.hevce_session_ssim.restype = ctypes.c_int
+        L.hevce_session_ssim.argtypes = [ctypes.c_void_p, ctypes.c_int, _dp]
         L.hevce_set_devices.restype = ctypes.c_int
         L.hevce_set_devices.argtypes = [ctypes.c_int, _ip]
         L.hevce_set_max_dim.restype = ctypes.c_int
@@ -89,7 +96,8 @@ def lib():
         L.hevce_session_download_decoded.argtypes = [ctypes.c_void_p, ctypes.POINTER(_u8p)]
         L.hevce_session_partition.restype = ctypes.c_int
         L.hevce_session_partition.argtypes = [ctypes.c_void_p, ctypes.c_int, _u8p, _u8p, _u8p]
-        for f in ("hevce_session_kernel_ms", "hevce_session_commit_ms", "hevce_session_quality_ms", "hevce_session_deblock_ms"):
+        for f in ("hevce_session_kernel_ms", "hevce_session_commit_ms", "hevce_session_quality_ms", "hevce_session_deblock_ms",
+                  "hevce_session_ssim_ms"):
             getattr(L, f).restype = ctypes.c_float
             getattr(L, f).argtypes = [ctypes.c_void_p]
         for f in ("hevce_session_launches", "hevce_session_grid"):
@@ -210,6 +218,35 @@ def HEVCImageEncoderBatchDecoded(imgs, qpd6, outputs=None):
     return [outs[i][: lens[i]].tobytes() for i in range(n)], rcons, decs
 
 
+def HEVCImageEncoderBatchTarget(imgs, target, metric="ssim", decoded=False):
+    """Each picture at the coarsest qpd6 whose decoded picture meets `target` (scalar or one per picture): SSIM
+    (metric="ssim", hevce_session_ssim of the decoded picture) or PSNR in dB (metric="psnr").  The search rule is that of
+    include/hevce.h; a picture no qpd6 satisfies gets qpd6 0, and its quality shows it missed the target.
+    Returns (streams, recons, qpd6, quality), with the decoded pictures after recons when decoded=True."""
+    metrics = {"psnr": METRIC_PSNR, "ssim": METRIC_SSIM}
+    if metric not in metrics:
+        raise HevceError(ERR_ARG, f"HEVCImageEncoderBatchTarget: metric must be one of {sorted(metrics)}")
+    imgs = [np.ascontiguousarray(i, dtype=np.uint8) for i in imgs]
+    n = len(imgs)
+    tg = np.full(n, float(target)) if np.isscalar(target) else np.ascontiguousarray(target, dtype=np.float64)
+    if tg.shape != (n,):
+        raise HevceError(ERR_ARG, "HEVCImageEncoderBatchTarget: one target per picture")
+    outs, rcons = _out_buffers([i.shape for i in imgs], get_max_dim())
+    decs = [np.zeros_like(r) for r in rcons] if decoded else None
+    ys = (ctypes.c_int * n)(*[i.shape[0] for i in imgs])
+    xs = (ctypes.c_int * n)(*[i.shape[1] for i in imgs])
+    qs = np.zeros(n, np.int32)
+    qual = np.zeros(n, np.float64)
+    lens = (ctypes.c_int * n)()
+    dp = ctypes.POINTER(ctypes.c_double)
+    rc = lib().HEVCImageEncoderBatchTarget(n, _ptr_array(outs), _ptr_array(imgs), _ptr_array(rcons), _ptr_array(decs) if decoded else None,
+                                           ys, xs, metrics[metric], tg.ctypes.data_as(dp), qs.ctypes.data_as(_ip), qual.ctypes.data_as(dp), lens)
+    if rc < 0:
+        raise HevceError(rc, "HEVCImageEncoderBatchTarget")
+    streams = [outs[i][: lens[i]].tobytes() for i in range(n)]
+    return (streams, rcons, decs, qs, qual) if decoded else (streams, rcons, qs, qual)
+
+
 def set_devices(ordinals):
     arr = (ctypes.c_int * len(ordinals))(*ordinals)
     rc = lib().hevce_set_devices(len(ordinals), arr)
@@ -323,6 +360,19 @@ class Session:
         if rc < 0:
             raise HevceError(rc, "hevce_session_decoded_quality")
         return mse, psnr
+
+    def ssim(self, decoded=False):
+        """Mean SSIM of every picture, reduced on the device: the coded picture (the source padded by edge replication)
+        against the reconstruction of the last encode, or with decoded=True against the decoded picture after deblock()."""
+        out = np.zeros(self.n, np.float64)
+        rc = lib().hevce_session_ssim(self._h, 1 if decoded else 0, out.ctypes.data_as(ctypes.POINTER(ctypes.c_double)))
+        if rc < 0:
+            raise HevceError(rc, "hevce_session_ssim")
+        return out
+
+    @property
+    def ssim_ms(self):
+        return lib().hevce_session_ssim_ms(self._h)
 
     def partition(self, i):
         """Decisions of picture i: (cu_size, mode) per 4x4 unit and kind per 8x8 unit (0 one TU, 1 four TUs, 2 NxN)."""

@@ -63,6 +63,33 @@ HEVCE_API int HEVCImageEncoderBatchDecoded(int n, unsigned char *const *pbuffers
                           unsigned char *const *img_rcons, unsigned char *const *img_decs, int *ysz, int *xsz,
                           const int *qpd6, int *stream_len);
 
+/*
+ * New: encode each picture at the coarsest qpd6 whose decoded picture meets a quality target.
+ *   metric    HEVCE_METRIC_PSNR: dB of the decoded picture (hevce_session_decoded_quality);
+ *             HEVCE_METRIC_SSIM: SSIM of the decoded picture (hevce_session_ssim with decoded = 1)
+ *   target    n values; a probe meets target[i] when its quality >= target[i]
+ *   qpd6      out: the chosen qpd6 of each picture
+ *   quality   out (may be NULL): the chosen probe's quality
+ *   img_decs  NULL, or n buffers that receive the decoded pictures as in HEVCImageEncoderBatchDecoded
+ * Search rule, per picture (quality is not assumed to be monotone in qpd6; the result is what this rule picks):
+ *     lo, hi = -1, 5
+ *     while hi - lo > 1:
+ *         q = (lo + hi) / 2                   -- the first probe is 2
+ *         if quality(q) >= target: lo = q else: hi = q
+ *     chosen = lo >= 0 ? lo : 0               -- every chosen value has been probed
+ * A picture takes at most three probes (2, 3, 4 or 2, 0, 1), so the call runs at most three rounds of the batch path of
+ * HEVCImageEncoderBatch, each over the pictures still searching at their probe qpd6.  pbuffers, img_rcons, img_decs,
+ * stream_len, qpd6 and quality receive the chosen probe's results.  A target no setting meets gives qpd6 0 and its
+ * quality (the call still returns 0; the caller sees quality < target).  A NaN target, another metric or any argument
+ * HEVCImageEncoderBatch rejects is HEVCE_ERR_ARG before any device work.  ysz / xsz are written back once, at the end,
+ * as in HEVCImageEncoderBatch, and are left as they were on failure.  returns 0, or a negative HEVCE_ERR_*.
+ */
+#define HEVCE_METRIC_PSNR 0
+#define HEVCE_METRIC_SSIM 1
+HEVCE_API int HEVCImageEncoderBatchTarget(int n, unsigned char *const *pbuffers, const unsigned char *const *imgs,
+                          unsigned char *const *img_rcons, unsigned char *const *img_decs, int *ysz, int *xsz,
+                          int metric, const double *target, int *qpd6, double *quality, int *stream_len);
+
 /* ---- extensions used by the benchmark harness and the multi-process launcher ------------------------------ */
 
 /* Restrict the library to `count` CUDA device ordinals (default: every visible device; the environment
@@ -123,6 +150,16 @@ HEVCE_API int   hevce_session_deblock(hevce_session *s);
 HEVCE_API float hevce_session_deblock_ms(const hevce_session *s);   /* CUDA-event duration of that hevce_deblock_kernel launch */
 HEVCE_API int   hevce_session_download_decoded(hevce_session *s, unsigned char *const *img_decs);   /* HBM -> host */
 HEVCE_API int   hevce_session_decoded_quality(hevce_session *s, double *mse, double *psnr);
+/* f7: per-picture mean SSIM, reduced on the device, with scikit-image's defaults as HEVCeval.py calls it: uniform 7x7
+ * window, sample covariance, K1 = 0.01, K2 = 0.03, data_range = 256, mean over the (H-6) x (W-6) window centres inside
+ * the picture.  It compares two planes at the padded size H x W: the coded picture, src[min(y, ysz-1)][min(x, xsz-1)],
+ * which for a picture inside the size limit is the source padded by edge replication, and (decoded = 0) the
+ * reconstruction or (decoded = 1) the decoded picture.  PSNR keeps its definition over the area both cover.  ssim: n
+ * doubles.  HEVCE_ERR_STATE before the first hevce_session_encode (decoded = 0) or unless hevce_session_deblock has
+ * run since the last configure, upload or encode (decoded = 1).  A picture's value is bit-identical however it is
+ * batched. */
+HEVCE_API int   hevce_session_ssim(hevce_session *s, int decoded, double *ssim);
+HEVCE_API float hevce_session_ssim_ms(const hevce_session *s);   /* CUDA-event duration of the last SSIM launch (both kernels) */
 HEVCE_API long long hevce_session_h2d_bytes(const hevce_session *s);
 HEVCE_API long long hevce_session_d2h_bytes(const hevce_session *s);
 HEVCE_API void hevce_session_destroy(hevce_session *s);
